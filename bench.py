@@ -3,7 +3,7 @@
 Benchmark of the threshold-Paillier hot path on B200 (BASELINE.json metric: threshold
 decrypts/sec at 2048-bit N).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
     python bench.py --split --gpus N [--config cfg2|cfg3] [--total T]   # ONE process, one fixed batch
                                                                         # sharded over N GPUs (strong scaling)
 
@@ -223,6 +223,24 @@ class ClockSampler:
             out.update(sm_mhz=clocks[len(clocks) // 2], sm_max_mhz=mx, reasons=sorted(reasons),
                        samples=len(clocks), power_w_max=max(power) if power else None)
         return out
+
+
+DUMP_ROWS = 8192   # ciphertexts --dump-outputs writes: 3 x 8192 x 128 partial limbs + plaintexts = 30 MB as float64
+
+
+def dump_outputs(out_dir: str, partials, plaintexts, status) -> None:
+    """What the timed call returned in its last step, as float64 arrays of the 32-bit limb values
+    (exact): partials [shares, rows, n2_limbs], plaintexts [rows, n_limbs] and status [shares + 1,
+    rows] (per party, then the combination; 0 = ok), for a fixed seeded sample of the batch (all of
+    it up to DUMP_ROWS ciphertexts) whose row indices go to rows.npy."""
+    import numpy as np
+
+    B = plaintexts.shape[0]
+    rows = np.arange(B) if B <= DUMP_ROWS else np.sort(np.random.default_rng(2024).choice(B, DUMP_ROWS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("rows", rows), ("partials", partials[:, rows]), ("plaintexts", plaintexts[rows]),
+                      ("status", status[:, rows])):
+        np.save(os.path.join(out_dir, name + ".npy"), arr.astype(np.float64))
 
 
 def cpu_baseline(dk, cores: int, sample: int, seed: int, cpython: bool = True) -> dict:
@@ -636,7 +654,14 @@ def main() -> None:
     ap.add_argument("--split", action="store_true", help="one process, one fixed batch sharded over --gpus devices (strong scaling)")
     ap.add_argument("--config", default="cfg2", choices=["cfg2", "cfg3"], help="--split: which BASELINE.json configuration")
     ap.add_argument("--total", type=int, default=0, help="--split: ciphertexts in the batch (0 = two waves per GPU)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one returned (partials, plaintexts, status of "
+                         "a fixed sample of rank 0's ciphertexts) as DIR/<name>.npy, float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.split):
+        ap.error("--dump-outputs: only the default (device-resident threshold decryption) path writes its outputs")
 
     if args.impl == "reference":
         run_reference(args)
@@ -788,6 +813,8 @@ def main() -> None:
             x = x * limbs_to_ints(part_host[s, i : i + 1])[0] % n2
         assert (x - 1) % dk.n == 0, "combined value minus one not divisible by N"
         assert limbs_to_ints(plain_host[i : i + 1])[0] == ((x - 1) // dk.n) * theta_inv % dk.n, "combine mismatch"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, part_host, plain_host, d_status.cpu().numpy().reshape(shares + 1, B))
 
     # ---- end to end through the public host-buffer call ------------------------------------------
     e2e = None
@@ -806,7 +833,7 @@ def main() -> None:
             _native.check(_native.lib.dkg_threshold_decrypt_batch(
                 tctx._h, np_cts.ctypes.data, pinned_plain.data_ptr(), pinned_partials.data_ptr(), pinned_status.data_ptr(), B))
 
-        e2e_steps = max(1, min(args.steps, 3))
+        e2e_steps = args.steps
         e2e_step()
         barrier()
         t0 = time.perf_counter()

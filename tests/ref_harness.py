@@ -1,11 +1,13 @@
 """
 Test harness that runs the REFERENCE's own ``DistributedPaillier`` / ``PaillierSharedKey`` code in
-one process: where the unmodified reference is importable (``baseline/_ref``, the pip ``--target``
-install recorded in DESIGN.md -- it travels to the GPU box -- or ``/root/reference/src`` on the
-build container), its un-vendored third-party imports are satisfied by the data-holder shims in
-``tests/golden/ref_shims`` and the parties talk through the in-process ``FakePool`` below instead
-of ``tno.mpc.communication``'s HTTP pool (API used by the reference: ``async_broadcast``,
-``recv_all``; ``distributed_keygen.py:357-370, 476-496``).  Test infrastructure only.
+one process: where the unmodified reference is importable (``baseline/_ref``, the git-ignored pip
+``--target`` install recorded in DESIGN.md, or the ``src`` directory of a checkout of the reference
+named by ``DKG_REFERENCE_SRC``), its un-vendored third-party imports are satisfied by the
+data-holder shims in ``tests/golden/ref_shims`` and the parties talk through the in-process
+``FakePool`` below instead of ``tno.mpc.communication``'s HTTP pool (API used by the reference:
+``async_broadcast``, ``recv_all``; ``distributed_keygen.py:357-370, 476-496``).  The repository
+does not contain the reference: without a copy, the tests that use this harness skip.  Test
+infrastructure only.
 """
 from __future__ import annotations
 
@@ -18,13 +20,13 @@ from typing import Any
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIMS = os.path.join(ROOT, "tests", "golden", "ref_shims")
-CANDIDATES = [os.path.join(ROOT, "baseline", "_ref"), "/root/reference/src"]
+CANDIDATES = [os.path.join(ROOT, "baseline", "_ref"), os.environ.get("DKG_REFERENCE_SRC")]
 
 
 def import_reference() -> Any:
     """The reference package, or ``None`` when no copy of it is reachable from here."""
     for path in CANDIDATES:
-        if os.path.isdir(os.path.join(path, "tno", "mpc", "protocols", "distributed_keygen")):
+        if path and os.path.isdir(os.path.join(path, "tno", "mpc", "protocols", "distributed_keygen")):
             for extra in (SHIMS, path):
                 if extra not in sys.path:
                     sys.path.insert(0, extra)

@@ -8,6 +8,8 @@ import ctypes
 import os
 import random
 import re
+import subprocess
+import sys
 
 import pytest
 
@@ -26,17 +28,28 @@ def test_library_exports_every_declared_symbol():
     assert _native.lib.dkg_version() >= 100
 
 
-def test_no_cpu_fallback_without_device():
-    import protocols.distributed_keygen_b200 as eng
-    from protocols.distributed_keygen_b200 import _native
+_NO_DEVICE_CHECK = """
+import sys
+sys.path.insert(0, sys.argv[1])
+import pytest
+import protocols.distributed_keygen_b200 as eng
+from protocols.distributed_keygen_b200 import _native
 
-    if _native.device_count() > 0:
-        pytest.skip("a CUDA device is present")
-    with pytest.raises(_native.DkgError) as err:
-        eng.ModexpContext(35, 3)
-    assert err.value.code == _native.DKG_ERR_CUDA
-    with pytest.raises(_native.DkgError):
-        eng.modexp_grouped([35], [3], [[2]])
+assert _native.device_count() == 0
+with pytest.raises(_native.DkgError) as err:
+    eng.ModexpContext(35, 3)
+assert err.value.code == _native.DKG_ERR_CUDA
+with pytest.raises(_native.DkgError):
+    eng.modexp_grouped([35], [3], [[2]])
+"""
+
+
+def test_no_cpu_fallback_without_device():
+    """Runs in a child process with every device hidden (CUDA_VISIBLE_DEVICES empty), so that the
+    no-device path is also checked on machines that have a GPU."""
+    res = subprocess.run([sys.executable, "-c", _NO_DEVICE_CHECK, ROOT], capture_output=True, text=True,
+                         env={**os.environ, "CUDA_VISIBLE_DEVICES": ""})
+    assert res.returncode == 0, res.stderr
 
 
 def test_argument_validation():

@@ -21,7 +21,7 @@ import pytest
 import ref_harness as rh
 
 REF = rh.import_reference()
-needs_ref = pytest.mark.skipif(REF is None, reason="no copy of the reference reachable (baseline/_ref or /root/reference)")
+needs_ref = pytest.mark.skipif(REF is None, reason="no copy of the reference reachable (baseline/_ref or $DKG_REFERENCE_SRC)")
 
 PLAINTEXTS = [1, 2, 3, -1, -2, -3, 1.5, 42.42424242, -1.5, -42.42424242]   # ref: test_distributed_keygen.py:21-23
 

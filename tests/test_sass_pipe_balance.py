@@ -7,11 +7,22 @@ inside their noinline Montgomery product (the target of their CALLs)."""
 from __future__ import annotations
 
 import collections
+import os
 import re
 import shutil
 import subprocess
 
 import pytest
+
+
+def _cuobjdump() -> str | None:
+    """cuobjdump from PATH, else from the CUDA toolkit ($CUDA_HOME, /usr/local/cuda)."""
+    for path in (shutil.which("cuobjdump"), *(os.path.join(h, "bin", "cuobjdump") for h in
+                                              (os.environ.get("CUDA_HOME", ""), "/usr/local/cuda") if h)):
+        if path and os.access(path, os.X_OK):
+            return path
+    return None
+
 
 KERNELS = [("_ZN3dkg17modexp_nsq_kernelILi13ELi5ELb0EEEvNS_9NsqParamsE", 13),
            ("_ZN3dkg23modexp_nsq_multi_kernelILi13ELi5ELb0EEEvNS_14NsqMultiParamsE", 13),
@@ -23,9 +34,10 @@ KERNELS = [("_ZN3dkg17modexp_nsq_kernelILi13ELi5ELb0EEEvNS_9NsqParamsE", 13),
 def test_hot_montgomery_product_keeps_the_multiplier_pipe_for_multiplies(KERNEL, K):
     from protocols.distributed_keygen_b200 import _native
 
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
-    sass = subprocess.run(["cuobjdump", "-sass", "-fun", KERNEL, _native.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    cuobjdump = _cuobjdump()
+    if cuobjdump is None:
+        pytest.skip("cuobjdump not found (PATH, $CUDA_HOME/bin, /usr/local/cuda/bin)")
+    sass = subprocess.run([cuobjdump, "-sass", "-fun", KERNEL, _native.LIB_PATH], capture_output=True, text=True, check=True).stdout
     insts = [(int(m.group(1), 16), m.group(2)) for m in re.finditer(r"/\*([0-9a-f]{4,6})\*/\s+(?:@!?U?P\d+\s+)?([A-Z0-9_.]+)", sass)]
     assert len(insts) > 5000, "kernel not found in the library"
     targets = collections.Counter(int(t, 16) for t in re.findall(r"CALL\.REL\.NOINC\s+0x([0-9a-f]+)", sass))
