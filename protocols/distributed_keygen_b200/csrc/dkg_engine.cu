@@ -8,6 +8,7 @@
 #include <atomic>
 #include <mutex>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../../include/dkg_b200.h"
@@ -20,6 +21,7 @@
 #include "dkg_nsq_params_fwd.h"
 #include "dkg_nsq_io.cuh"
 #include "dkg_coop_params.h"
+#include "dkg_kernel_table.h"
 
 namespace {
 
@@ -47,8 +49,6 @@ constexpr Shape kShapes[] = {
     {20, 13}, {16, 17},
 };
 
-using KernelFn = void (*)(const dkg::ModexpParams);
-
 // A CTA-uniform constant in the layout of a lane-private operand ([vector][lane], vectors of
 // VW = 4 limbs when K % 4 == 0, else 2): multiplication operands are always read with this
 // one stride (see WarpIO in dkg_modexp.cuh), so constants that get multiplied are replicated.
@@ -60,28 +60,6 @@ void append_lane_replicated(std::vector<uint32_t>& out, const std::vector<uint32
 }
 }  // namespace
 namespace dkg {
-// one per dkg_kernels_<n>.cu
-KernelFn lookup_kernel_group0(int, int); KernelFn lookup_kernel_group1(int, int);
-KernelFn lookup_kernel_group2(int, int); KernelFn lookup_kernel_group3(int, int);
-KernelFn lookup_kernel_group4(int, int); KernelFn lookup_kernel_group5(int, int);
-using BatchInvFn = void (*)(const BatchInvParams);
-BatchInvFn lookup_batchinv_group0(int, int); BatchInvFn lookup_batchinv_group1(int, int);
-BatchInvFn lookup_batchinv_group2(int, int); BatchInvFn lookup_batchinv_group3(int, int);
-BatchInvFn lookup_batchinv_group4(int, int); BatchInvFn lookup_batchinv_group5(int, int);
-using NsqFn = void (*)(const NsqParams);
-NsqFn lookup_nsq_group0(int, int); NsqFn lookup_nsq_group1(int, int); NsqFn lookup_nsq_group2(int, int);
-NsqFn lookup_nsq_group3(int, int); NsqFn lookup_nsq_group4(int, int); NsqFn lookup_nsq_group5(int, int);
-NsqFn lookup_nsq_bg_group0(int, int); NsqFn lookup_nsq_bg_group1(int, int); NsqFn lookup_nsq_bg_group2(int, int);
-NsqFn lookup_nsq_bg_group3(int, int); NsqFn lookup_nsq_bg_group4(int, int); NsqFn lookup_nsq_bg_group5(int, int);
-using NsqMultiFn = void (*)(const NsqMultiParams);
-NsqMultiFn lookup_nsq_multi_bg_group0(int, int); NsqMultiFn lookup_nsq_multi_bg_group1(int, int); NsqMultiFn lookup_nsq_multi_bg_group2(int, int);
-NsqMultiFn lookup_nsq_multi_bg_group3(int, int); NsqMultiFn lookup_nsq_multi_bg_group4(int, int); NsqMultiFn lookup_nsq_multi_bg_group5(int, int);
-NsqMultiFn lookup_nsq_multi_group0(int, int); NsqMultiFn lookup_nsq_multi_group1(int, int); NsqMultiFn lookup_nsq_multi_group2(int, int);
-NsqMultiFn lookup_nsq_multi_group3(int, int); NsqMultiFn lookup_nsq_multi_group4(int, int); NsqMultiFn lookup_nsq_multi_group5(int, int);
-using GroupedFn = void (*)(const GroupedParams);
-GroupedFn lookup_grouped_group0(int, int); GroupedFn lookup_grouped_group1(int, int);
-GroupedFn lookup_grouped_group2(int, int); GroupedFn lookup_grouped_group3(int, int);
-GroupedFn lookup_grouped_group4(int, int); GroupedFn lookup_grouped_group5(int, int);
 void launch_group_setup(const GroupedParams& p, cudaStream_t stream);
 // dkg_coop.cu: the cooperative (warp-per-operand) latency kernels
 int coop_max_warps(int K, bool pair_kernel);
@@ -91,21 +69,13 @@ cudaError_t launch_coop_combine(int K, const CoopCombineParams& p, int ctas, int
 }  // namespace dkg
 namespace {
 
-KernelFn lookup_kernel(int K, int M) {
-  KernelFn (*groups[])(int, int) = {dkg::lookup_kernel_group0, dkg::lookup_kernel_group1, dkg::lookup_kernel_group2,
-                                    dkg::lookup_kernel_group3, dkg::lookup_kernel_group4, dkg::lookup_kernel_group5};
-  for (auto g : groups)
-    if (KernelFn f = g(K, M)) return f;
-  return nullptr;
-}
-
-dkg::BatchInvFn lookup_batchinv(int K, int M) {
-  dkg::BatchInvFn (*groups[])(int, int) = {dkg::lookup_batchinv_group0, dkg::lookup_batchinv_group1,
-                                           dkg::lookup_batchinv_group2, dkg::lookup_batchinv_group3,
-                                           dkg::lookup_batchinv_group4, dkg::lookup_batchinv_group5};
-  for (auto g : groups)
-    if (dkg::BatchInvFn f = g(K, M)) return f;
-  return nullptr;
+// every kernel compiled for shape (K, M), whichever dkg_kernels_<n>.cu holds it
+dkg::ShapeKernels lookup_kernels(int K, int M) {
+  dkg::ShapeKernels k;
+  for (auto g : {dkg::find_kernels_group0, dkg::find_kernels_group1, dkg::find_kernels_group2,
+                 dkg::find_kernels_group3, dkg::find_kernels_group4, dkg::find_kernels_group5})
+    g(K, M, &k);
+  return k;
 }
 
 bool pick_shape(int limbs, Shape* out) {
@@ -323,7 +293,7 @@ struct dkg_modexp_ctx {
   size_t smem = 0;
   size_t scratch_per_warp = 0;
   size_t scratch_q_offset = 0;
-  KernelFn kernel = nullptr;
+  dkg::KernelFn kernel = nullptr;
   dkg::BatchInvFn inv_kernel = nullptr;
   int inv_warps = 1;
   size_t inv_smem = 0;
@@ -348,42 +318,27 @@ struct dkg_modexp_ctx {
   uint32_t* d_cconsts = nullptr;   // kernel constants (CoopNsqParams::consts)
   uint32_t* d_cio = nullptr;       // entry/exit constants for cLc
   dkg::CoopPlanTable cfull{}, clow{};
-  bool use_nsq = true;             // knobs read once, when the context is created
-  bool use_batch_inverse = true;
   bool ct_table = false;           // constant-time table access (masked scan of all entries)
 };
 
 namespace {
 
-int choose_window(int ebits, int max_w = 6) {
-  if (const char* f = getenv("DKG_FORCE_WINDOW")) {  // tuning/debug knob
-    int w = atoi(f);
-    if (w >= 1 && w <= max_w) return w;
-  }
+// Window width 1..max_w of least cost(ebits, w), in multiplications (the narrowest on a tie).
+int choose_window(int ebits, int max_w, double (*cost)(int ebits, int w)) {
   int best = 1;
-  long best_cost = -1;
-  for (int w = 1; w <= max_w; ++w) {
-    long cost = ((1L << w) - 2) + (ebits + w - 1) / w;
-    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = w; }
-  }
+  for (int w = 2; w <= max_w; ++w)
+    if (cost(ebits, w) < cost(ebits, best)) best = w;
   return best;
 }
 
-// Window width under constant-time table access: every multiplication scans all 2^w entries
-// (~0.034 of a multiplication's time per entry at 2048-bit N: 560 B per thread against the L2/HBM
-// share of a thread), so narrower windows win: cost = 2^w - 2 + ceil(E/w) * (1 + 0.034 * 2^w).
-int choose_window_ct(int ebits) {
-  if (const char* f = getenv("DKG_FORCE_WINDOW")) {
-    int w = atoi(f);
-    if (w >= 1 && w <= 7) return w;
-  }
-  int best = 1;
-  double best_cost = -1;
-  for (int w = 1; w <= 7; ++w) {
-    const double cost = (double)((1L << w) - 2) + (double)((ebits + w - 1) / w) * (1.0 + 0.034 * (double)(1L << w));
-    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = w; }
-  }
-  return best;
+// Fixed windows: 2^w - 2 multiplications build the table, then one per digit.
+double fixed_window_cost(int ebits, int w) { return (double)(((1L << w) - 2) + (ebits + w - 1) / w); }
+
+// Constant-time table access: every multiplication scans all 2^w entries (~0.034 of a
+// multiplication's time per entry at 2048-bit N: 560 B per thread against the L2/HBM share of a
+// thread), so narrower windows win: cost = 2^w - 2 + ceil(E/w) * (1 + 0.034 * 2^w).
+double ct_window_cost(int ebits, int w) {
+  return (double)((1L << w) - 2) + (double)((ebits + w - 1) / w) * (1.0 + 0.034 * (double)(1L << w));
 }
 
 // Sliding windows for the fixed-exponent contexts.  The exponent belongs to the key, so the whole
@@ -394,19 +349,7 @@ int choose_window_ct(int ebits) {
 // and means "start from table[idx]".
 constexpr uint32_t kOpNoMul = 0xffu;
 constexpr uint32_t kOpMulOne = 0xfeu;  // fixed windows: digit 0 multiplies by the Montgomery one
-int choose_sliding_window(int ebits) {
-  if (const char* f = getenv("DKG_FORCE_WINDOW")) {  // tuning/debug knob
-    int w = atoi(f);
-    if (w >= 1 && w <= 7) return w;
-  }
-  int best = 1;
-  long best_cost = -1;
-  for (int w = 1; w <= 7; ++w) {
-    long cost = (1L << (w - 1)) + ebits / (w + 1);
-    if (best_cost < 0 || cost < best_cost) { best_cost = cost; best = w; }
-  }
-  return best;
-}
+double sliding_window_cost(int ebits, int w) { return (double)((1L << (w - 1)) + ebits / (w + 1)); }
 std::vector<uint32_t> sliding_window_ops(const uint32_t* e, int ebits, int w, int* table_entries, int* nmul) {
   auto bit = [&](int i) { return (e[i / 32] >> (i % 32)) & 1u; };
   std::vector<uint32_t> ops;
@@ -433,17 +376,9 @@ std::vector<uint32_t> sliding_window_ops(const uint32_t* e, int ebits, int w, in
   return ops;
 }
 
-int launch_modexp_nsq(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status,
-                      size_t count, cudaStream_t stream, bool* handled, const uint32_t* d_mrows = nullptr, int m_limbs = 0,
-                      const unsigned int** redo_flag = nullptr);
-int launch_modexp_coop(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status, size_t count,
-                       cudaStream_t stream, bool* handled, const uint32_t* d_mrows, int m_limbs);
-
 // Chain warps of the batched inversion: chains of 32 groups keep the binary-GCD count at 1/32 of
 // the elements but leave most SMs idle (56 warps for a 56 832-element launch); the chain products
 // dominate, so spread them over every SM as long as a chain keeps at least 4 groups.
-int inversion_chain_warps(const DeviceState* d, const dkg_modexp_ctx* ctx, unsigned long long ngroups);
-
 int inversion_chain_warps(const DeviceState* d, const dkg_modexp_ctx* ctx, unsigned long long ngroups) {
   unsigned long long nchain = (ngroups + 31) / 32;
   const unsigned long long wide = std::min<unsigned long long>((unsigned long long)d->sm_count * std::max(ctx->inv_warps, 1), ngroups / 4);
@@ -451,73 +386,77 @@ int inversion_chain_warps(const DeviceState* d, const dkg_modexp_ctx* ctx, unsig
   return (int)std::max<unsigned long long>(nchain, 1);
 }
 
-int launch_modexp_inner(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status,
-                        const uint32_t* d_final_mul, size_t count, cudaStream_t stream);
+// Batched inversion of `count` rows modulo ctx's modulus: Montgomery's trick along chains of ~32
+// groups, one binary-GCD inversion per chain lane.  Its work area is the start of d->aux,
+//   chain_s | chain_p | scratch | chain_status | any_bad (32 words),
+// and callers put their own buffers behind it.  Returns its size in words; with `b`, also lays it
+// out there (d->aux must already be that large).
+size_t batchinv_area(const dkg_modexp_ctx* ctx, size_t count, dkg::BatchInvParams* b = nullptr) {
+  const DeviceState* d = ctx->dev;
+  const unsigned long long ngroups = (count + 31) / 32;
+  const size_t gwords = (size_t)ctx->Lp * 32;
+  const int nchain = inversion_chain_warps(d, ctx, ngroups);
+  if (b) {
+    b->chain_s = d->aux; b->chain_p = d->aux + ngroups * gwords; b->scratch = d->aux + 2 * ngroups * gwords;
+    b->chain_status = b->scratch + (size_t)nchain * gwords;
+    b->any_bad = reinterpret_cast<unsigned int*>(b->chain_status + (size_t)nchain * 32);
+    b->nchain_warps = nchain; b->chain_len = (int)((ngroups + nchain - 1) / nchain);
+  }
+  return 2 * ngroups * gwords + (size_t)nchain * gwords + (size_t)nchain * 32 + 32;
+}
+
+// Launches the batched inversion of `rows` in the area above.  plain_out null: the inverses stay in
+// chain_s (Montgomery form, lane layout) for the direct kernel, which takes *b.  Otherwise they go
+// there as canonical rows (`rows` itself is fine: a chain warp reads all its groups before it writes
+// any), and *b->any_bad is set on the device if a chain met a non-unit.
+int launch_batchinv(dkg_modexp_ctx* ctx, const uint32_t* rows, size_t count, uint32_t* plain_out, cudaStream_t stream,
+                    dkg::BatchInvParams* b) {
+  *b = dkg::BatchInvParams{};
+  batchinv_area(ctx, count, b);
+  b->bases = rows; b->count = count; b->in_limbs = ctx->limbs; b->consts = ctx->d_consts; b->n0inv = ctx->n0inv;
+  b->plain_out = plain_out;
+  if (plain_out) CUDA_TRY(cudaMemsetAsync(b->any_bad, 0, sizeof(unsigned int), stream));
+  else b->any_bad = nullptr;
+  const int blocks = (b->nchain_warps + ctx->inv_warps - 1) / ctx->inv_warps;
+  ctx->inv_kernel<<<blocks, ctx->inv_warps * 32, ctx->inv_smem, stream>>>(*b);
+  CUDA_TRY(cudaGetLastError());
+  g_launches.fetch_add(1);
+  return DKG_OK;
+}
+
+// CTAs of a wave launch of ctas x warps warps: fewer when the batch has fewer groups of 32 rows
+int wave_ctas(int ctas, int warps, size_t count) {
+  const unsigned long long ngroups = (count + 31) / 32;
+  return ngroups < (unsigned long long)ctas * warps ? (int)((ngroups + warps - 1) / warps) : ctas;
+}
+
+// The direct kernel (dkg_modexp.cuh) on `count` rows.  inv: batched inversion of the bases to take
+// instead of inverting each one, or null; run_if: device flag that predicates the launch, or null.
+int launch_direct(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status,
+                  const uint32_t* d_final_mul, size_t count, cudaStream_t stream, const dkg::BatchInvParams* inv,
+                  const unsigned int* run_if) {
+  DeviceState* d = ctx->dev;
+  int rc = ensure_scratch(d, (size_t)ctx->ctas * ctx->warps * ctx->scratch_per_warp);
+  if (rc != DKG_OK) return rc;
+  CUDA_TRY(cudaMemsetAsync(d->counter, 0, sizeof(unsigned int), stream));
+  dkg::ModexpParams p{};
+  if (inv) { p.inv_mont = inv->chain_s; p.chain_status = inv->chain_status; p.nchain_warps = inv->nchain_warps; }
+  p.bases = d_bases; p.out = d_out; p.status = d_status; p.count = count; p.in_limbs = ctx->limbs;
+  p.consts = ctx->d_consts; p.ops = ctx->d_ops; p.nops = ctx->nops; p.tab_entries = ctx->tab_entries; p.table_odd = ctx->table_odd;
+  p.negative = ctx->negative; p.n0inv = ctx->n0inv; p.scratch = d->scratch;
+  p.scratch_per_warp = ctx->scratch_per_warp; p.scratch_q_offset = ctx->scratch_q_offset; p.counter = d->counter; p.final_mul = d_final_mul;
+  p.run_if = run_if;
+  ctx->kernel<<<wave_ctas(ctx->ctas, ctx->warps, count), ctx->warps * 32, ctx->smem, stream>>>(p);
+  CUDA_TRY(cudaGetLastError());
+  g_launches.fetch_add(1);
+  return DKG_OK;
+}
 
 // out-of-range rows (>= modulus) are flagged and zeroed after the compute kernels
 int launch_range_check(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status, size_t count,
                        cudaStream_t stream) {
   const unsigned blocks = (unsigned)((count * 32 + 255) / 256);
   dkg::range_check_kernel<<<blocks, 256, 0, stream>>>(d_bases, ctx->d_consts, ctx->limbs, count, d_out, d_status);
-  CUDA_TRY(cudaGetLastError());
-  g_launches.fetch_add(1);
-  return DKG_OK;
-}
-
-int launch_modexp(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status,
-                  const uint32_t* d_final_mul, size_t count, cudaStream_t stream) {
-  if (count == 0) return DKG_OK;
-  int rc = launch_modexp_inner(ctx, d_bases, d_out, d_status, d_final_mul, count, stream);
-  if (rc != DKG_OK) return rc;
-  return launch_range_check(ctx, d_bases, d_out, d_status, count, stream);
-}
-
-int launch_modexp_inner(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status,
-                        const uint32_t* d_final_mul, size_t count, cudaStream_t stream) {
-  if (count == 0) return DKG_OK;
-  DeviceState* d = ctx->dev;
-  CUDA_TRY(cudaSetDevice(d->device));
-  const unsigned int* redo_flag = nullptr;
-  if (ctx->nsq && d_final_mul == nullptr && ctx->use_nsq) {
-    bool handled = false;
-    int rc0 = launch_modexp_nsq(ctx, d_bases, d_out, d_status, count, stream, &handled, nullptr, 0, &redo_flag);
-    if (rc0 != DKG_OK || (handled && redo_flag == nullptr)) return rc0;
-    // handled with a device-side "redo" flag: fall through to the direct kernel, predicated on it
-  }
-  const unsigned long long ngroups = (count + 31) / 32;
-  const int total_warps = ctx->ctas * ctx->warps;
-  int ctas = ctx->ctas;
-  if (ngroups < (unsigned long long)total_warps) ctas = (int)((ngroups + ctx->warps - 1) / ctx->warps);
-  int rc = ensure_scratch(d, (size_t)total_warps * ctx->scratch_per_warp);
-  if (rc != DKG_OK) return rc;
-  CUDA_TRY(cudaMemsetAsync(d->counter, 0, sizeof(unsigned int), stream));
-  dkg::ModexpParams p{};
-  if (ctx->negative && ctx->inv_kernel != nullptr && ngroups >= 2 && ctx->use_batch_inverse && redo_flag == nullptr) {
-    // Montgomery's trick along chains of ~32 groups: one binary-GCD inversion per chain lane
-    // (the predicated redo of a pair-path call inverts per element instead: exact status)
-    const size_t gwords = (size_t)ctx->Lp * 32;
-    const int nchain = inversion_chain_warps(d, ctx, ngroups);
-    const int chain_len = (int)((ngroups + nchain - 1) / nchain);
-    const size_t words = 2 * ngroups * gwords + (size_t)nchain * gwords + (size_t)nchain * 32;
-    rc = ensure_aux(d, words);
-    if (rc != DKG_OK) return rc;
-    dkg::BatchInvParams b{};
-    b.bases = d_bases; b.count = count; b.in_limbs = ctx->limbs; b.consts = ctx->d_consts; b.n0inv = ctx->n0inv;
-    b.chain_s = d->aux; b.chain_p = d->aux + ngroups * gwords; b.scratch = d->aux + 2 * ngroups * gwords;
-    b.chain_status = b.scratch + (size_t)nchain * gwords;
-    b.nchain_warps = nchain; b.chain_len = chain_len;
-    const int blocks = (nchain + ctx->inv_warps - 1) / ctx->inv_warps;
-    ctx->inv_kernel<<<blocks, ctx->inv_warps * 32, ctx->inv_smem, stream>>>(b);
-    CUDA_TRY(cudaGetLastError());
-    g_launches.fetch_add(1);
-    p.inv_mont = b.chain_s; p.chain_status = b.chain_status; p.nchain_warps = nchain;
-  }
-  p.bases = d_bases; p.out = d_out; p.status = d_status; p.count = count; p.in_limbs = ctx->limbs;
-  p.consts = ctx->d_consts; p.ops = ctx->d_ops; p.nops = ctx->nops; p.tab_entries = ctx->tab_entries; p.table_odd = ctx->table_odd;
-  p.negative = ctx->negative; p.n0inv = ctx->n0inv; p.scratch = d->scratch;
-  p.scratch_per_warp = ctx->scratch_per_warp; p.scratch_q_offset = ctx->scratch_q_offset; p.counter = d->counter; p.final_mul = d_final_mul;
-  p.run_if = redo_flag;
-  ctx->kernel<<<ctas, ctx->warps * 32, ctx->smem, stream>>>(p);
   CUDA_TRY(cudaGetLastError());
   g_launches.fetch_add(1);
   return DKG_OK;
@@ -577,120 +516,138 @@ int launch_modexp_coop_parties(dkg_modexp_ctx* const* parties, int nparties, con
   return DKG_OK;
 }
 
-int launch_modexp_coop(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status, size_t count,
-                       cudaStream_t stream, bool* handled, const uint32_t* d_mrows, int m_limbs) {
-  int rc = launch_modexp_coop_parties(&ctx, 1, d_bases, d_out, d_status, count, stream, d_mrows, m_limbs);
-  *handled = rc == DKG_OK;
-  return rc;
-}
-
-// Modulus N^2 with known N: [batched inversion ->] entry (pairs) -> pair exponentiation -> exit.
-// Falls back to the direct kernel (handled = false) when a chain of the batched inversion hit a
-// non-unit, so that the per-element status comes out exact.
-int launch_modexp_nsq(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status,
-                      size_t count, cudaStream_t stream, bool* handled, const uint32_t* d_mrows, int m_limbs,
-                      const unsigned int** redo_flag) {
+// Modulus N^2 with known N: entry (pairs) -> pair exponentiation -> exit, from `src` (the bases, or
+// their batched inversion) through `pairs` (count * 2 nLp words) to d_out.
+int launch_pair(dkg_modexp_ctx* ctx, const uint32_t* src, uint32_t* pairs, uint32_t* d_out, uint8_t* d_status,
+                size_t count, cudaStream_t stream, const uint32_t* d_mrows, int m_limbs) {
   DeviceState* d = ctx->dev;
-  *handled = false;
-  const unsigned int* no_flag = nullptr;
-  if (redo_flag == nullptr) redo_flag = &no_flag;
-  *redo_flag = nullptr;
-  if (ctx->coop && count <= ctx->coop_max) return launch_modexp_coop(ctx, d_bases, d_out, d_status, count, stream, handled, d_mrows, m_limbs);
-  const unsigned long long ngroups = (count + 31) / 32;
-  const int Lp = ctx->nLp;
-  const size_t pair_words = count * (size_t)(2 * Lp);
-  const uint32_t* src = d_bases;
-  size_t inv_words = 0, inv_off = 0;
-  const bool inv_in_kernel = ctx->negative && ctx->nsq_inv;
-  if (ctx->negative && !inv_in_kernel) {
-    if (ctx->inv_kernel == nullptr || ngroups < 1) return DKG_OK;  // let the direct kernel do it
-    const size_t gwords = (size_t)ctx->Lp * 32;
-    const int nchain = inversion_chain_warps(d, ctx, ngroups);
-    const int chain_len = (int)((ngroups + nchain - 1) / nchain);
-    inv_words = 2 * ngroups * gwords + (size_t)nchain * gwords + (size_t)nchain * 32 + 32 + count * (size_t)ctx->limbs;
-    int rc = ensure_aux(d, inv_words + pair_words);
-    if (rc != DKG_OK) return rc;
-    dkg::BatchInvParams b{};
-    b.bases = d_bases; b.count = count; b.in_limbs = ctx->limbs; b.consts = ctx->d_consts; b.n0inv = ctx->n0inv;
-    b.chain_s = d->aux; b.chain_p = d->aux + ngroups * gwords; b.scratch = d->aux + 2 * ngroups * gwords;
-    b.chain_status = b.scratch + (size_t)nchain * gwords;
-    b.any_bad = reinterpret_cast<unsigned int*>(b.chain_status + (size_t)nchain * 32);
-    b.plain_out = b.chain_status + (size_t)nchain * 32 + 32;
-    b.nchain_warps = nchain; b.chain_len = chain_len;
-    CUDA_TRY(cudaMemsetAsync(b.any_bad, 0, sizeof(unsigned int), stream));
-    const int blocks = (nchain + ctx->inv_warps - 1) / ctx->inv_warps;
-    ctx->inv_kernel<<<blocks, ctx->inv_warps * 32, ctx->inv_smem, stream>>>(b);
-    CUDA_TRY(cudaGetLastError());
-    g_launches.fetch_add(1);
-    // No host round trip: if a chain met a non-unit (any_bad != 0, decided on the device) the pair
-    // path's results of this call are discarded and the direct kernel -- launched below on the same
-    // stream, predicated on that flag -- redoes the call with the exact per-element status.
-    *redo_flag = b.any_bad;
-    src = b.plain_out;
-    inv_off = inv_words;
-  } else {
-    int rc = ensure_aux(d, pair_words);
-    if (rc != DKG_OK) return rc;
-  }
-  uint32_t* pairs = d->aux + inv_off;
-  const int total_warps = ctx->ctas * ctx->nwarps;
-  int ctas = ctx->ctas;
-  if (ngroups < (unsigned long long)total_warps) ctas = (int)((ngroups + ctx->nwarps - 1) / ctx->nwarps);
-  int rc = ensure_scratch(d, (size_t)total_warps * ctx->nscratch_per_warp);
+  int rc = ensure_scratch(d, (size_t)ctx->ctas * ctx->nwarps * ctx->nscratch_per_warp);
   if (rc != DKG_OK) return rc;
   dkg::NsqIoParams e{};
-  e.in = src; e.out = pairs; e.count = count; e.io_limbs = ctx->limbs; e.Lp = Lp; e.consts = ctx->d_nio; e.n0inv = ctx->n_n0inv;
+  e.in = src; e.out = pairs; e.count = count; e.io_limbs = ctx->limbs; e.Lp = ctx->nLp; e.consts = ctx->d_nio; e.n0inv = ctx->n_n0inv;
   e.mrows = nullptr; e.m_limbs = 0;
   dkg::nsq_entry_kernel<<<(unsigned)((count + 63) / 64), 64, 0, stream>>>(e);
   CUDA_TRY(cudaMemsetAsync(d->counter, 0, sizeof(unsigned int), stream));
   dkg::NsqParams q{};
   q.pairs_in = pairs; q.pairs_out = pairs; q.count = count; q.consts = ctx->d_nconsts; q.ops = ctx->d_ops;
   q.nops = ctx->nops; q.tab_entries = ctx->tab_entries; q.table_odd = ctx->table_odd; q.ct_table = ctx->ct_table ? 1 : 0; q.scratch = d->scratch; q.scratch_per_warp = ctx->nscratch_per_warp;
-  q.negative = inv_in_kernel ? 1 : 0; q.status = d_status; q.inv_slot = ctx->ninv_slot;
+  q.negative = ctx->negative && ctx->nsq_inv ? 1 : 0; q.status = d_status; q.inv_slot = ctx->ninv_slot;
   if (d_status) CUDA_TRY(cudaMemsetAsync(d_status, 0, count, stream));
   q.scratch_q_offset = ctx->nscratch_q_offset; q.counter = d->counter;
   {
     KernelTimer kt(d, stream);
-    ctx->nsq_kernel<<<ctas, ctx->nwarps * 32, ctx->nsmem, stream>>>(q);
+    ctx->nsq_kernel<<<wave_ctas(ctx->ctas, ctx->nwarps, count), ctx->nwarps * 32, ctx->nsmem, stream>>>(q);
   }
   dkg::NsqIoParams x = e;
   x.in = pairs; x.out = d_out; x.mrows = d_mrows; x.m_limbs = m_limbs;
   dkg::nsq_exit_kernel<<<(unsigned)((count + 63) / 64), 64, 0, stream>>>(x);
   CUDA_TRY(cudaGetLastError());
   g_launches.fetch_add(3);
-  *handled = true;
   return DKG_OK;
 }
 
-dkg::NsqFn lookup_nsq(int K, int M) {
-  dkg::NsqFn (*groups[])(int, int) = {dkg::lookup_nsq_group0, dkg::lookup_nsq_group1, dkg::lookup_nsq_group2,
-                                      dkg::lookup_nsq_group3, dkg::lookup_nsq_group4, dkg::lookup_nsq_group5};
-  for (auto g : groups)
-    if (dkg::NsqFn f = g(K, M)) return f;
-  return nullptr;
+// How one fixed-exponent call runs (pick_route decides from the context and the batch size):
+enum class Route {
+  coop,       // N^2 context, batch <= coop_max: entry -> cooperative pair kernel -> exit
+  pair,       // N^2 context, positive exponent or in-kernel inversion: entry -> pair kernel -> exit
+  pair_redo,  // N^2 context, negative exponent: batched inversion -> pair route -> direct kernel if
+              // a chain of the inversion met a non-unit, so that the per-element status comes out exact
+  direct,     // anything else: [batched inversion ->] direct kernel
+};
+
+Route pick_route(const dkg_modexp_ctx* ctx, size_t count) {
+  if (!ctx->nsq) return Route::direct;
+  if (ctx->coop && count <= ctx->coop_max) return Route::coop;
+  if (!ctx->negative || ctx->nsq_inv) return Route::pair;
+  return ctx->inv_kernel ? Route::pair_redo : Route::direct;
 }
 
-dkg::NsqFn lookup_nsq_bg(int K, int M) {
-  dkg::NsqFn (*groups[])(int, int) = {dkg::lookup_nsq_bg_group0, dkg::lookup_nsq_bg_group1, dkg::lookup_nsq_bg_group2,
-                                      dkg::lookup_nsq_bg_group3, dkg::lookup_nsq_bg_group4, dkg::lookup_nsq_bg_group5};
-  for (auto g : groups)
-    if (dkg::NsqFn f = g(K, M)) return f;
-  return nullptr;
-}
-dkg::NsqMultiFn lookup_nsq_multi(int K, int M, bool bg) {
-  dkg::NsqMultiFn (*plain[])(int, int) = {dkg::lookup_nsq_multi_group0, dkg::lookup_nsq_multi_group1, dkg::lookup_nsq_multi_group2,
-                                          dkg::lookup_nsq_multi_group3, dkg::lookup_nsq_multi_group4, dkg::lookup_nsq_multi_group5};
-  dkg::NsqMultiFn (*wide[])(int, int) = {dkg::lookup_nsq_multi_bg_group0, dkg::lookup_nsq_multi_bg_group1, dkg::lookup_nsq_multi_bg_group2,
-                                         dkg::lookup_nsq_multi_bg_group3, dkg::lookup_nsq_multi_bg_group4, dkg::lookup_nsq_multi_bg_group5};
-  auto& groups = bg ? wide : plain;
-  for (auto g : groups)
-    if (dkg::NsqMultiFn f = g(K, M)) return f;
-  return nullptr;
+// Encryption's factor (1 + m N): m rows folded into the exit kernel of the pair routes, whole rows
+// multiplied in by the direct kernel.
+struct EncryptFactor { const uint32_t* m; int m_limbs; const uint32_t* final_mul; };
+
+// One fixed-exponent call on `count` device rows by its route, then the range check (which
+// encryption's pair routes skip).
+int launch_modexp(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32_t* d_out, uint8_t* d_status, size_t count,
+                  cudaStream_t stream, const EncryptFactor* enc = nullptr) {
+  if (count == 0) return DKG_OK;
+  DeviceState* d = ctx->dev;
+  CUDA_TRY(cudaSetDevice(d->device));
+  const Route route = pick_route(ctx, count);
+  const uint32_t* mrows = enc ? enc->m : nullptr;
+  const int m_limbs = enc ? enc->m_limbs : 0;
+  dkg::BatchInvParams inv{};
+  int rc = DKG_OK;
+  if (route == Route::coop) {
+    rc = launch_modexp_coop_parties(&ctx, 1, d_bases, d_out, d_status, count, stream, mrows, m_limbs);
+  } else if (route == Route::direct) {
+    const bool batched = ctx->negative && ctx->inv_kernel != nullptr && count > 32;   // >= 2 groups
+    if (batched) rc = ensure_aux(d, batchinv_area(ctx, count));
+    if (rc == DKG_OK && batched) rc = launch_batchinv(ctx, d_bases, count, nullptr, stream, &inv);
+    if (rc == DKG_OK)
+      rc = launch_direct(ctx, d_bases, d_out, d_status, enc ? enc->final_mul : nullptr, count, stream, batched ? &inv : nullptr, nullptr);
+  } else if (route == Route::pair) {
+    rc = ensure_aux(d, count * (size_t)(2 * ctx->nLp));
+    if (rc == DKG_OK) rc = launch_pair(ctx, d_bases, d->aux, d_out, d_status, count, stream, mrows, m_limbs);
+  } else {
+    // aux: inversion area | canonical inverses | pairs.  No host round trip: the redo is predicated
+    // on the device-side any_bad, and discards the pair route's results when it runs.
+    const size_t inv_words = batchinv_area(ctx, count), plain_words = count * (size_t)ctx->limbs;
+    rc = ensure_aux(d, inv_words + plain_words + count * (size_t)(2 * ctx->nLp));
+    uint32_t* plain = d->aux + inv_words;
+    if (rc == DKG_OK) rc = launch_batchinv(ctx, d_bases, count, plain, stream, &inv);
+    if (rc == DKG_OK) rc = launch_pair(ctx, plain, plain + plain_words, d_out, d_status, count, stream, mrows, m_limbs);
+    if (rc == DKG_OK) rc = launch_direct(ctx, d_bases, d_out, d_status, nullptr, count, stream, nullptr, inv.any_bad);
+  }
+  if (rc != DKG_OK || (enc && route != Route::direct)) return rc;
+  return launch_range_check(ctx, d_bases, d_out, d_status, count, stream);
 }
 
 // shapes for the pair components, in order of preference per padded width
 constexpr Shape kNsqShapes[] = {{4, 1}, {4, 2}, {4, 3}, {8, 2}, {6, 3}, {12, 2}, {16, 2}, {12, 3}, {16, 3},
                                 {16, 4}, {13, 5}, {14, 5}, {12, 6}, {16, 5}, {16, 6}, {14, 7}, {12, 11}, {16, 9}};
+
+// Constants of the pair arithmetic modulo N (dkg_nsq.cuh, dkg_coop.cuh) for R = 2^(32 L), dense on
+// L limbs; a residue c mod N^2 is the pair (c mod N, (c div N) * R mod N).  n, n2: N and N^2.
+struct PairConsts {
+  dkg_host::Limbs N, ninv, dneg, r2a, r2b, onea, oneb, twoa, twob, plain1, zero;   // ninv: -N^-1 mod 2^(32 K)
+  dkg_host::Limbs r2, ninvpos;   // entry / exit: R^2 mod N, N^-1 mod R
+};
+PairConsts pair_consts(const dkg_host::Limbs& n, const dkg_host::Limbs& n2, int L, int K) {
+  using dkg_host::Limbs;
+  PairConsts c;
+  c.N.assign(L, 0);
+  std::copy(n.begin(), n.end(), c.N.begin());
+  c.ninv = dkg_host::neg_inv_block(c.N, K);
+  c.ninvpos = dkg_host::negate(dkg_host::neg_inv_block(c.N, L));
+  const Limbs r = dkg_host::pow2_mod((size_t)32 * L, c.N);
+  c.r2 = dkg_host::pow2_mod((size_t)64 * L, c.N);
+  c.dneg.assign(L, 0);   // -R mod N
+  if (std::any_of(r.begin(), r.end(), [](uint32_t w) { return w != 0; })) { c.dneg = c.N; dkg_host::sub_inplace(c.dneg, r); }
+  // pairs of R^2 mod N^2 and R mod N^2: g = g0 + g1 N  ->  (g0, g1 * R mod N)
+  auto plain_pair = [&](size_t pow2bits, Limbs* pa, Limbs* pb) {
+    Limbs q, g0;
+    dkg_host::divmod_slow(dkg_host::pow2_mod(pow2bits, n2), n, &q, &g0);
+    pa->assign(L, 0);
+    std::copy(g0.begin(), g0.end(), pa->begin());
+    Limbs g1(L, 0);
+    for (int i = 0; i < (int)q.size() && i < L; ++i) g1[i] = q[i];
+    *pb = dkg_host::mulmod_slow(g1, r, c.N);
+  };
+  plain_pair((size_t)64 * L, &c.r2a, &c.r2b);
+  plain_pair((size_t)32 * L, &c.onea, &c.oneb);
+  c.plain1.assign(L, 0);
+  c.plain1[0] = 1;
+  c.zero.assign(L, 0);
+  // pair of 2 with 2N added to its a component (Newton step of pair_invert): (2 onea + 2N, 2 oneb - 2R mod N)
+  c.twoa.assign(L, 0);
+  uint64_t carry = 0;
+  for (int i = 0; i < L; ++i) { uint64_t t = (uint64_t)c.onea[i] + c.N[i] + carry; c.twoa[i] = (uint32_t)t; carry = t >> 32; }
+  uint32_t c2 = 0;
+  for (int i = 0; i < L; ++i) { const uint32_t nc = c.twoa[i] >> 31; c.twoa[i] = (c.twoa[i] << 1) | c2; c2 = nc; }
+  c.twob = dkg_host::submod(dkg_host::addmod(c.oneb, c.oneb, c.N), dkg_host::addmod(r, r, c.N), c.N);
+  return c;
+}
 
 }  // namespace
 
@@ -769,9 +726,8 @@ int dkg_modexp_ctx_create(int device, const uint32_t* modulus, int mod_limbs, co
   ctx->shape = shape;
   ctx->Lp = shape.K * shape.M;
   ctx->negative = exp_negative ? 1 : 0;
-  ctx->use_nsq = getenv("DKG_NO_NSQ") == nullptr;   // environment knobs are read here, once per context
-  ctx->use_batch_inverse = getenv("DKG_NO_BATCH_INVERSE") == nullptr;
-  ctx->kernel = lookup_kernel(shape.K, shape.M);
+  const dkg::ShapeKernels kernels = lookup_kernels(shape.K, shape.M);
+  ctx->kernel = kernels.fixed;
   if (!ctx->kernel) { delete ctx; return fail(DKG_ERR_UNSUPPORTED, "kernel shape not compiled"); }
 
   const int Lp = ctx->Lp, K = shape.K;
@@ -800,11 +756,11 @@ int dkg_modexp_ctx_create(int device, const uint32_t* modulus, int mod_limbs, co
   std::vector<uint32_t> ops;
   ctx->ct_table = ct_table_setting();
   if (const char* sw = getenv("DKG_SLIDING_WINDOW"); sw && atoi(sw) != 0 && !ctx->ct_table) {
-    ctx->wbits = choose_sliding_window(ctx->ebits);
+    ctx->wbits = choose_window(ctx->ebits, 7, sliding_window_cost);
     ops = sliding_window_ops(exponent, ctx->ebits, ctx->wbits, &ctx->tab_entries, &ctx->nmul);
     ctx->table_odd = 1;
   } else {
-    ctx->wbits = ctx->ct_table ? choose_window_ct(ctx->ebits) : choose_window(ctx->ebits, 7);
+    ctx->wbits = choose_window(ctx->ebits, 7, ctx->ct_table ? ct_window_cost : fixed_window_cost);
     const int ndigits = (ctx->ebits + ctx->wbits - 1) / ctx->wbits;
     for (int t = 0; t < ndigits; ++t) {
       const int lowbit = ctx->wbits * (ndigits - 1 - t);
@@ -835,7 +791,7 @@ int dkg_modexp_ctx_create(int device, const uint32_t* modulus, int mod_limbs, co
   ctx->scratch_q_offset = std::max<size_t>(tsize, 4) * (size_t)Lp * 32;
   ctx->scratch_per_warp = ctx->scratch_q_offset + (size_t)Lp * 32;
 
-  ctx->inv_kernel = lookup_batchinv(shape.K, shape.M);
+  ctx->inv_kernel = kernels.batchinv;
   {
     const size_t inv_per_warp = (size_t)6 * Lp * 32 * 4;
     ctx->inv_warps = (int)std::min<size_t>(2, (kMaxDynSmem - uni) / inv_per_warp);
@@ -881,18 +837,8 @@ int dkg_modexp_ctx_create_nsq(int device, const uint32_t* n, int n_limbs, const 
   while (ln > 1 && n[ln - 1] == 0) --ln;
   if ((n[0] & 1u) == 0) return fail(DKG_ERR_INVALID, "modulus must be odd");
   // N^2 and the ordinary context on it (constants for the batched inversion and the fallback)
-  dkg_host::Limbs nn(n, n + ln), n2(2 * ln, 0);
-  for (int i = 0; i < ln; ++i) {
-    uint64_t carry = 0;
-    for (int j = 0; j < ln; ++j) {
-      uint64_t t = (uint64_t)nn[i] * nn[j] + n2[i + j] + carry;
-      n2[i + j] = (uint32_t)t;
-      carry = t >> 32;
-    }
-    n2[i + ln] = (uint32_t)carry;
-  }
-  int l2 = 2 * ln;
-  while (l2 > 1 && n2[l2 - 1] == 0) --l2;
+  const dkg_host::Limbs nn(n, n + ln), n2 = dkg_host::square(nn);
+  const int l2 = (int)n2.size();
   dkg_modexp_ctx* ctx = nullptr;
   int rc = dkg_modexp_ctx_create(device, n2.data(), l2, exponent, exp_limbs, exp_negative, &ctx);
   if (rc != DKG_OK) return rc;
@@ -902,14 +848,10 @@ int dkg_modexp_ctx_create_nsq(int device, const uint32_t* n, int n_limbs, const 
   if (nbits < 2) return DKG_OK;  // N = 1: nothing to gain
   const int need = (nbits + 3 + 31) / 32;
   Shape sh{};
-  dkg::NsqFn kernel = nullptr;
-  if (const char* f = getenv("DKG_NSQ_SHAPE")) {  // tuning knob: "K,M"
-    int k = 0, m = 0;
-    if (sscanf(f, "%d,%d", &k, &m) == 2 && k * m >= need && (kernel = lookup_nsq(k, m)) != nullptr) sh = Shape{k, m};
-  }
-  if (!kernel)
-    for (const Shape& c : kNsqShapes)
-      if (c.K * c.M >= need && (kernel = lookup_nsq(c.K, c.M)) != nullptr) { sh = c; break; }
+  dkg::ShapeKernels kernels;
+  for (const Shape& c : kNsqShapes)
+    if (c.K * c.M >= need && (kernels = lookup_kernels(c.K, c.M)).nsq != nullptr) { sh = c; break; }
+  dkg::NsqFn kernel = kernels.nsq;
   if (!kernel || sh.K * sh.M > dkg::kNsqMaxL) return DKG_OK;  // too wide: keep the direct kernel
   // Lp: limbs of the pair components, R = 2^(32 Lp).  In the kernel's memory a block of K limbs
   // occupies a slot of KP = K + (K & 1) limbs (whole 64-bit vectors; odd K: one zero pad limb), a
@@ -920,61 +862,19 @@ int dkg_modexp_ctx_create_nsq(int device, const uint32_t* n, int n_limbs, const 
     for (size_t i = 0; i < v.size(); ++i) out[(i / K) * KP + i % K] = v[i];
     return out;
   };
-  dkg_host::Limbs N(Lp, 0);
-  for (int i = 0; i < ln; ++i) N[i] = nn[i];
-  dkg_host::Limbs ninv = dkg_host::neg_inv_block(N, K);
-  dkg_host::Limbs ninv_full_neg = dkg_host::neg_inv_block(N, Lp), ninvpos(Lp);
-  {
-    uint64_t carry = 1;
-    for (int i = 0; i < Lp; ++i) { uint64_t t = (uint64_t)(~ninv_full_neg[i]) + carry; ninvpos[i] = (uint32_t)t; carry = t >> 32; }
-  }
-  dkg_host::Limbs r_mod_n = dkg_host::pow2_mod((size_t)32 * Lp, N);
-  dkg_host::Limbs r2_mod_n = dkg_host::pow2_mod((size_t)64 * Lp, N);
-  dkg_host::Limbs dneg(Lp, 0);  // -R mod N
-  {
-    bool zero = true;
-    for (uint32_t w : r_mod_n) zero = zero && (w == 0);
-    if (!zero) { dneg = N; dkg_host::sub_inplace(dneg, r_mod_n); }
-  }
-  // pairs of R^2 mod N^2 and R mod N^2: g = g0 + g1 N  ->  (g0, g1 * R mod N)
-  dkg_host::Limbs n2p(n2.begin(), n2.begin() + l2);
-  auto plain_pair = [&](size_t pow2bits, dkg_host::Limbs* pa, dkg_host::Limbs* pb) {
-    dkg_host::Limbs g = dkg_host::pow2_mod(pow2bits, n2p);     // l2 limbs
-    dkg_host::Limbs nshort(nn.begin(), nn.begin() + ln), qd, rd;
-    dkg_host::divmod_slow(g, nshort, &qd, &rd);
-    pa->assign(Lp, 0); pb->assign(Lp, 0);
-    for (int i = 0; i < ln; ++i) (*pa)[i] = rd[i];
-    dkg_host::Limbs g1(Lp, 0);
-    for (int i = 0; i < (int)qd.size() && i < Lp; ++i) g1[i] = qd[i];
-    *pb = dkg_host::mulmod_slow(g1, r_mod_n, N);
-  };
-  dkg_host::Limbs r2a, r2b, onea, oneb;
-  plain_pair((size_t)64 * Lp, &r2a, &r2b);
-  plain_pair((size_t)32 * Lp, &onea, &oneb);
-  dkg_host::Limbs plain1(Lp, 0), zero(Lp, 0);
-  plain1[0] = 1;
+  const PairConsts pc = pair_consts(nn, n2, Lp, K);
   std::vector<uint32_t> kc;
-  for (const dkg_host::Limbs* v : {&N, &ninv, &dneg, &r2a, &r2b, &onea, &oneb, &plain1, &zero}) {
+  for (const dkg_host::Limbs* v : {&pc.N, &pc.ninv, &pc.dneg, &pc.r2a, &pc.r2b, &pc.onea, &pc.oneb, &pc.plain1, &pc.zero}) {
     const dkg_host::Limbs sv = slotted(*v);
     kc.insert(kc.end(), sv.begin(), sv.end());
   }
-  for (const dkg_host::Limbs* v : {&r2a, &r2b, &onea, &oneb, &plain1, &zero}) append_lane_replicated(kc, slotted(*v), KP);
-  // pair of 2 with 2N added to its a component (Newton step of pair_invert): (2 onea + 2N, 2 oneb - 2R mod N)
-  {
-    dkg_host::Limbs twoa(Lp, 0);
-    uint64_t carry = 0;
-    for (int i = 0; i < Lp; ++i) { uint64_t t = (uint64_t)onea[i] + N[i] + carry; twoa[i] = (uint32_t)t; carry = t >> 32; }
-    uint32_t c2 = 0;
-    for (int i = 0; i < Lp; ++i) { const uint32_t nc = twoa[i] >> 31; twoa[i] = (twoa[i] << 1) | c2; c2 = nc; }
-    const dkg_host::Limbs b2 = dkg_host::addmod(oneb, oneb, N), rr = dkg_host::addmod(r_mod_n, r_mod_n, N);
-    const dkg_host::Limbs twob = dkg_host::submod(b2, rr, N);
-    for (const dkg_host::Limbs* v : {(const dkg_host::Limbs*)&twoa, &twob}) {
-      const dkg_host::Limbs sv = slotted(*v);
-      kc.insert(kc.end(), sv.begin(), sv.end());
-    }
+  for (const dkg_host::Limbs* v : {&pc.r2a, &pc.r2b, &pc.onea, &pc.oneb, &pc.plain1, &pc.zero}) append_lane_replicated(kc, slotted(*v), KP);
+  for (const dkg_host::Limbs* v : {&pc.twoa, &pc.twob}) {
+    const dkg_host::Limbs sv = slotted(*v);
+    kc.insert(kc.end(), sv.begin(), sv.end());
   }
   std::vector<uint32_t> ioc;
-  for (const dkg_host::Limbs* v : {&N, &r2_mod_n, &ninvpos}) ioc.insert(ioc.end(), v->begin(), v->end());
+  for (const dkg_host::Limbs* v : {&pc.N, &pc.r2, &pc.ninvpos}) ioc.insert(ioc.end(), v->begin(), v->end());
 
   const size_t uni = (((size_t)(2 * Ls + KP + Lp) * 4 + 15) / 16) * 16 +
                      (((size_t)dkg::sched_total_words_closed(sh.M) * 4 + 15) / 16) * 16;  // consts | schedule table
@@ -984,12 +884,10 @@ int dkg_modexp_ctx_create_nsq(int device, const uint32_t* n, int n_limbs, const 
   // wide keys: shared memory, not registers, caps the warps per SM; with fewer than 10 take the
   // variant that keeps the b component in global scratch (a only in shared memory)
   bool bg = false;
-  if (warps < 10 && env_long("DKG_NSQ_BG", 1) != 0) {
-    if (dkg::NsqFn kb = lookup_nsq_bg(sh.K, sh.M)) {
-      kernel = kb; bg = true;
-      per_warp = (size_t)Ls * 32 * 4;
-      warps = (int)std::min<size_t>(maxw, (kMaxDynSmem - uni) / per_warp);
-    }
+  if (warps < 10 && env_long("DKG_NSQ_BG", 1) != 0 && kernels.nsq_bg != nullptr) {
+    kernel = kernels.nsq_bg; bg = true;
+    per_warp = (size_t)Ls * 32 * 4;
+    warps = (int)std::min<size_t>(maxw, (kMaxDynSmem - uni) / per_warp);
   }
   if (warps < 1) return DKG_OK;
   // window table (odd powers, then the slot of c^2 / the constant-time spare), then 4 pair slots of
@@ -1014,57 +912,18 @@ int dkg_modexp_ctx_create_nsq(int device, const uint32_t* n, int n_limbs, const 
     return fail(DKG_ERR_CUDA, std::string("nsq context: ") + cudaGetErrorString(e));
   }
   ctx->nshape = sh; ctx->nLp = Lp; ctx->nLs = Ls; ctx->nwarps = warps; ctx->nsmem = uni + per_warp * warps;
-  ctx->n_n0inv = ninv[0]; ctx->nsq_kernel = kernel; ctx->nsq = true;
+  ctx->n_n0inv = pc.ninv[0]; ctx->nsq_kernel = kernel; ctx->nsq = true;
 
   // ---- cooperative (warp-per-operand) latency path, dkg_coop.cuh: its own R = 2^(32 cLc) >= 8N -----
   int cK = 0, cnb = 0;
   const size_t coop_max = coop_limit(g_coop_max, "DKG_COOP_MAX", kCoopMaxDefault);
   if (coop_max > 0 && coop_shape(need, &cK, &cnb) && cK * cnb <= dkg::kNsqMaxL) {
     const int Lc = cK * cnb;
-    dkg_host::Limbs Nc(Lc, 0);
-    for (int i = 0; i < ln; ++i) Nc[i] = nn[i];
-    dkg_host::Limbs ni_c = dkg_host::neg_inv_block(Nc, Lc);
-    dkg_host::Limbs ninvpos_c(Lc);
-    {
-      uint64_t carry = 1;
-      for (int i = 0; i < Lc; ++i) { uint64_t t = (uint64_t)(~ni_c[i]) + carry; ninvpos_c[i] = (uint32_t)t; carry = t >> 32; }
-    }
-    dkg_host::Limbs r_c = dkg_host::pow2_mod((size_t)32 * Lc, Nc), r2_c = dkg_host::pow2_mod((size_t)64 * Lc, Nc);
-    dkg_host::Limbs dneg_c(Lc, 0);
-    {
-      bool zero_r = true;
-      for (uint32_t w : r_c) zero_r = zero_r && (w == 0);
-      if (!zero_r) { dneg_c = Nc; dkg_host::sub_inplace(dneg_c, r_c); }
-    }
-    auto plain_pair_c = [&](size_t pow2bits, dkg_host::Limbs* pa, dkg_host::Limbs* pb) {
-      dkg_host::Limbs g = dkg_host::pow2_mod(pow2bits, n2p);
-      dkg_host::Limbs nshort(nn.begin(), nn.begin() + ln), qd, rd;
-      dkg_host::divmod_slow(g, nshort, &qd, &rd);
-      pa->assign(Lc, 0);
-      for (int i = 0; i < ln; ++i) (*pa)[i] = rd[i];
-      dkg_host::Limbs g1(Lc, 0);
-      for (int i = 0; i < (int)qd.size() && i < Lc; ++i) g1[i] = qd[i];
-      *pb = dkg_host::mulmod_slow(g1, r_c, Nc);
-    };
-    dkg_host::Limbs cr2a, cr2b, conea, coneb;
-    plain_pair_c((size_t)64 * Lc, &cr2a, &cr2b);
-    plain_pair_c((size_t)32 * Lc, &conea, &coneb);
-    // constants of the Newton step of the in-kernel inversion: 2*ONE as (2 a + 2N, 2 b - 2R mod N)
-    dkg_host::Limbs twoa(Lc, 0), twob;
-    {
-      uint64_t carry = 0;
-      for (int i = 0; i < Lc; ++i) { uint64_t t = (uint64_t)conea[i] + Nc[i] + carry; twoa[i] = (uint32_t)t; carry = t >> 32; }
-      uint32_t c2 = 0;
-      for (int i = 0; i < Lc; ++i) { const uint32_t nc = twoa[i] >> 31; twoa[i] = (twoa[i] << 1) | c2; c2 = nc; }
-      const dkg_host::Limbs b2 = dkg_host::addmod(coneb, coneb, Nc), rr = dkg_host::addmod(r_c, r_c, Nc);
-      twob = dkg_host::submod(b2, rr, Nc);
-    }
-    dkg_host::Limbs cplain1(Lc, 0), czero(Lc, 0);
-    cplain1[0] = 1;
+    const PairConsts cp = pair_consts(nn, n2, Lc, Lc);
     std::vector<uint32_t> cc, cio;
-    for (const dkg_host::Limbs* v : {&Nc, &ni_c, &dneg_c, &cr2a, &cr2b, &conea, &coneb, &twoa, &twob, &cplain1, &czero})
+    for (const dkg_host::Limbs* v : {&cp.N, &cp.ninv, &cp.dneg, &cp.r2a, &cp.r2b, &cp.onea, &cp.oneb, &cp.twoa, &cp.twob, &cp.plain1, &cp.zero})
       cc.insert(cc.end(), v->begin(), v->end());
-    for (const dkg_host::Limbs* v : {&Nc, &r2_c, &ninvpos_c}) cio.insert(cio.end(), v->begin(), v->end());
+    for (const dkg_host::Limbs* v : {&cp.N, &cp.r2, &cp.ninvpos}) cio.insert(cio.end(), v->begin(), v->end());
     cudaError_t e2 = cudaMalloc(&ctx->d_cconsts, cc.size() * 4);
     if (e2 == cudaSuccess) e2 = cudaMalloc(&ctx->d_cio, cio.size() * 4);
     if (e2 == cudaSuccess) e2 = cudaMemcpy(ctx->d_cconsts, cc.data(), cc.size() * 4, cudaMemcpyHostToDevice);
@@ -1094,7 +953,7 @@ int dkg_modexp_batch_device(dkg_modexp_ctx* ctx, const uint32_t* d_bases, uint32
                             uint8_t* d_status, size_t count, void* stream) {
   if (!ctx || (count && (!d_bases || !d_out))) return fail(DKG_ERR_INVALID, "null argument");
   DeviceLease lease(ctx->dev, (cudaStream_t)stream);
-  return launch_modexp(ctx, d_bases, d_out, d_status, nullptr, count, (cudaStream_t)stream);
+  return launch_modexp(ctx, d_bases, d_out, d_status, count, (cudaStream_t)stream);
 }
 
 int dkg_modexp_batch(dkg_modexp_ctx* ctx, const uint32_t* bases, uint32_t* out, uint8_t* status,
@@ -1113,15 +972,13 @@ int dkg_modexp_batch(dkg_modexp_ctx* ctx, const uint32_t* bases, uint32_t* out, 
   if (e == cudaSuccess) e = bufs.alloc(&d_st, count);
   if (e != cudaSuccess) return fail(DKG_ERR_NOMEM, std::string("batch alloc: ") + cudaGetErrorString(e));
   CUDA_TRY(cudaMemcpyAsync(d_in, bases, bytes, cudaMemcpyHostToDevice, d->stream));
-  int rc = launch_modexp(ctx, d_in, d_out, d_st, nullptr, count, d->stream);
+  int rc = launch_modexp(ctx, d_in, d_out, d_st, count, d->stream);
   if (rc != DKG_OK) return rc;
   CUDA_TRY(cudaMemcpyAsync(out, d_out, bytes, cudaMemcpyDeviceToHost, d->stream));
   if (status) CUDA_TRY(cudaMemcpyAsync(status, d_st, count, cudaMemcpyDeviceToHost, d->stream));
   CUDA_TRY(cudaStreamSynchronize(d->stream));
   return DKG_OK;
 }
-
-// ---- not yet implemented entry points ------------------------------------------------------------
 
 }  // extern "C"
 
@@ -1182,27 +1039,11 @@ int dkg_combine_ctx_create(int device, const uint32_t* n, int n_limbs, const uin
   int rc = device_state(device, &dev);
   if (rc != DKG_OK) return rc;
   CUDA_TRY(cudaSetDevice(device));
-  // N^2 by schoolbook
-  dkg_host::Limbs nn(n, n + ln), n2(2 * ln, 0);
-  for (int i = 0; i < ln; ++i) {
-    uint64_t carry = 0;
-    for (int j = 0; j < ln; ++j) {
-      uint64_t t = (uint64_t)nn[i] * nn[j] + n2[i + j] + carry;
-      n2[i + j] = (uint32_t)t;
-      carry = t >> 32;
-    }
-    n2[i + ln] = (uint32_t)carry;
-  }
-  int l2 = 2 * ln;
-  while (l2 > 1 && n2[l2 - 1] == 0) --l2;
-  n2.resize(l2);
+  const dkg_host::Limbs nn(n, n + ln), n2 = dkg_host::square(nn);
+  const int l2 = (int)n2.size();
   dkg_host::Limbs rpow = dkg_host::pow2_mod((size_t)32 * l2 * shares, n2);
   dkg_host::Limbs ninvneg = dkg_host::neg_inv_block(nn, ln);
-  dkg_host::Limbs ninvpos(ln);
-  {
-    uint64_t carry = 1;
-    for (int i = 0; i < ln; ++i) { uint64_t t = (uint64_t)(~ninvneg[i]) + carry; ninvpos[i] = (uint32_t)t; carry = t >> 32; }
-  }
+  dkg_host::Limbs ninvpos = dkg_host::negate(ninvneg);
   dkg_host::Limbs th(ln, 0);
   for (int i = 0; i < ln && i < n_limbs; ++i) th[i] = theta_inv[i];
   if (!dkg_host::geq(nn, th) || th == nn) return fail(DKG_ERR_INVALID, "theta_inv must be < N");
@@ -1321,11 +1162,8 @@ extern "C" int dkg_encrypt_batch(dkg_modexp_ctx* ctx, const uint32_t* n, int n_l
     g_launches.fetch_add(1);
   }
   CUDA_TRY(cudaGetLastError());
-  int rc = DKG_OK;
-  bool handled = false;
-  if (ctx->nsq && ctx->use_nsq)  // r^N in pair arithmetic, (1 + m N) folded into the exit step
-    rc = launch_modexp_nsq(ctx, d_base, d_out, nullptr, count, d->stream, &handled, m ? d_m : nullptr, n_limbs);
-  if (rc == DKG_OK && !handled) rc = launch_modexp(ctx, d_base, d_out, nullptr, m ? d_fm : nullptr, count, d->stream);
+  const EncryptFactor enc{d_m, n_limbs, d_fm};
+  int rc = launch_modexp(ctx, d_base, d_out, nullptr, count, d->stream, &enc);
   if (rc != DKG_OK) return rc;
   CUDA_TRY(cudaMemcpyAsync(out, d_out, out_bytes, cudaMemcpyDeviceToHost, d->stream));
   CUDA_TRY(cudaStreamSynchronize(d->stream));
@@ -1333,17 +1171,6 @@ extern "C" int dkg_encrypt_batch(dkg_modexp_ctx* ctx, const uint32_t* n, int n_l
 }
 
 // ---- grouped modexp (biprimality test batch) -------------------------------------------------------
-namespace {
-dkg::GroupedFn lookup_grouped(int K, int M) {
-  dkg::GroupedFn (*groups[])(int, int) = {dkg::lookup_grouped_group0, dkg::lookup_grouped_group1,
-                                          dkg::lookup_grouped_group2, dkg::lookup_grouped_group3,
-                                          dkg::lookup_grouped_group4, dkg::lookup_grouped_group5};
-  for (auto g : groups)
-    if (dkg::GroupedFn f = g(K, M)) return f;
-  return nullptr;
-}
-}  // namespace
-
 namespace {
 
 struct GroupedPlan {
@@ -1356,7 +1183,7 @@ struct GroupedPlan {
 int plan_grouped(DeviceState* d, int limbs, int ebits, size_t count, GroupedPlan* plan) {
   if (const char* f = getenv("DKG_GROUPED_SHAPE")) {  // tuning knob: "K,M"
     int k = 0, m = 0;
-    if (sscanf(f, "%d,%d", &k, &m) == 2 && k * m >= limbs && (plan->kernel = lookup_grouped(k, m)) != nullptr) plan->shape = Shape{k, m};
+    if (sscanf(f, "%d,%d", &k, &m) == 2 && k * m >= limbs && (plan->kernel = lookup_kernels(k, m).grouped) != nullptr) plan->shape = Shape{k, m};
   }
   // by padded width, except that K = 22 (spills at 168 registers) yields to (14,5): measured
   // 304 k vs 222 k modexps/s on 65-limb candidates
@@ -1366,15 +1193,15 @@ int plan_grouped(DeviceState* d, int limbs, int ebits, size_t count, GroupedPlan
   };
   if (!plan->kernel)
     for (const Shape& sh : kGroupedPref)
-      if (sh.K * sh.M >= limbs && (plan->kernel = lookup_grouped(sh.K, sh.M)) != nullptr) { plan->shape = sh; break; }
+      if (sh.K * sh.M >= limbs && (plan->kernel = lookup_kernels(sh.K, sh.M).grouped) != nullptr) { plan->shape = sh; break; }
   if (!plan->kernel)
     for (const Shape& sh : kShapes)
-      if (sh.K * sh.M >= limbs && (plan->kernel = lookup_grouped(sh.K, sh.M)) != nullptr) { plan->shape = sh; break; }
+      if (sh.K * sh.M >= limbs && (plan->kernel = lookup_kernels(sh.K, sh.M).grouped) != nullptr) { plan->shape = sh; break; }
   if (!plan->kernel) return fail(DKG_ERR_UNSUPPORTED, "modulus wider than the grouped kernel shapes (132 limbs)");
   plan->Ka = plan->shape.K;
   plan->K = plan->shape.K + (plan->shape.K & 1);
   plan->Lp = plan->K * plan->shape.M;
-  plan->wbits = choose_window(ebits);
+  plan->wbits = choose_window(ebits, 6, fixed_window_cost);
   plan->ndigits = std::max(1, (ebits + plan->wbits - 1) / plan->wbits);
   const size_t per_warp_smem = ((size_t)2 * plan->Lp + plan->K) * 32 * 4;
   const size_t sched_bytes = (((size_t)dkg::sched_total_words_closed(plan->shape.M) * 4 + 15) / 16) * 16;
@@ -1384,9 +1211,7 @@ int plan_grouped(DeviceState* d, int limbs, int ebits, size_t count, GroupedPlan
   const size_t tsize = ((size_t)1 << plan->wbits) - 1;
   plan->q_off = std::max<size_t>(tsize, 1) * (size_t)plan->Lp * 32;
   plan->scratch_per_warp = plan->q_off + (size_t)3 * plan->Lp * 32;  // Q | R2 | ONER in lane layout
-  const unsigned long long nwork = (count + 31) / 32;
-  plan->ctas = d->sm_count;
-  if (nwork < (unsigned long long)plan->ctas * plan->warps) plan->ctas = (int)((nwork + plan->warps - 1) / plan->warps);
+  plan->ctas = wave_ctas(d->sm_count, plan->warps, count);
   int rc = ensure_scratch(d, (size_t)d->sm_count * plan->warps * plan->scratch_per_warp);
   if (rc != DKG_OK) return rc;
   cudaError_t e = cudaFuncSetAttribute((const void*)plan->kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan->smem);
@@ -1411,7 +1236,7 @@ bool plan_coop_grouped(DeviceState* d, const uint32_t* moduli, size_t groups, in
   const int need = (maxbits + 2 + 31) / 32;   // R >= 4N
   if (!coop_shape(need, &plan->K, &plan->nb)) return false;
   plan->Lc = plan->K * plan->nb;
-  plan->wbits = choose_window(ebits);
+  plan->wbits = choose_window(ebits, 6, fixed_window_cost);
   plan->ndigits = std::max(1, (ebits + plan->wbits - 1) / plan->wbits);
   coop_grid(d, plan->K, false, count, &plan->ctas, &plan->warps);
   plan->smem = (size_t)9 * plan->warps * plan->Lc * 4;
@@ -1435,10 +1260,26 @@ int launch_coop_grouped_batch(DeviceState* d, const CoopGroupedPlan& plan, const
   return DKG_OK;
 }
 
-// enqueue setup + grouped modexp on device buffers (gconsts/digits are caller-allocated scratch)
-int launch_grouped(DeviceState* d, const GroupedPlan& plan, const uint32_t* d_mod, const uint32_t* d_exp, int exp_limbs,
-                   const uint32_t* d_bases, uint32_t* d_out, size_t groups, int per_group, int limbs,
-                   uint32_t* d_gc, uint8_t* d_dig) {
+// Grouped modexp of groups x per_group device rows on d->stream: the cooperative kernel for small
+// batches, else group setup + wave kernel with per-group constants and digits allocated in `bufs`.
+// moduli, exps: host copies (the plans size themselves for the widest modulus and exponent).
+int launch_grouped(DeviceState* d, DevBufs& bufs, const uint32_t* moduli, const uint32_t* exps, const uint32_t* d_mod,
+                   const uint32_t* d_exp, int exp_limbs, const uint32_t* d_bases, uint32_t* d_out, size_t groups,
+                   int per_group, int limbs) {
+  int ebits = 0;
+  for (size_t g = 0; g < groups; ++g) ebits = std::max(ebits, dkg_host::bit_length(exps + g * (size_t)exp_limbs, exp_limbs));
+  const size_t count = groups * (size_t)per_group;
+  CoopGroupedPlan cplan;
+  if (plan_coop_grouped(d, moduli, groups, limbs, ebits, count, &cplan))
+    return launch_coop_grouped_batch(d, cplan, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, per_group, limbs);
+  GroupedPlan plan;
+  int rc = plan_grouped(d, limbs, ebits, count, &plan);
+  if (rc != DKG_OK) return rc;
+  uint32_t* d_gc;
+  uint8_t* d_dig;
+  cudaError_t e = bufs.alloc(&d_gc, groups * (size_t)(3 * plan.Lp + plan.K) * 4);
+  if (e == cudaSuccess) e = bufs.alloc(&d_dig, groups * (size_t)plan.ndigits);
+  if (e != cudaSuccess) return fail(DKG_ERR_NOMEM, std::string("grouped cudaMalloc: ") + cudaGetErrorString(e));
   CUDA_TRY(cudaMemsetAsync(d->counter, 0, sizeof(unsigned int), d->stream));
   dkg::GroupedParams p{};
   p.moduli = d_mod; p.exps = d_exp; p.bases = d_bases; p.out = d_out; p.groups = groups;
@@ -1466,33 +1307,20 @@ extern "C" int dkg_modexp_grouped(int device, const uint32_t* moduli, const uint
   int rc = device_state(device, &d);
   if (rc != DKG_OK) return rc;
   CUDA_TRY(cudaSetDevice(device));
-  int ebits = 0;
-  for (size_t g = 0; g < groups; ++g) ebits = std::max(ebits, dkg_host::bit_length(exps + g * (size_t)exp_limbs, exp_limbs));
   const size_t count = groups * (size_t)per_group;
   DeviceLease lease(d, d->stream);
-  CoopGroupedPlan cplan;
-  const bool coop = plan_coop_grouped(d, moduli, groups, limbs, ebits, count, &cplan);
-  GroupedPlan plan;
-  if (!coop) {
-    rc = plan_grouped(d, limbs, ebits, count, &plan);
-    if (rc != DKG_OK) return rc;
-  }
   DevBufs bufs(d->stream);
-  uint32_t *d_mod, *d_exp, *d_bases, *d_out, *d_gc = nullptr;
-  uint8_t* d_dig = nullptr;
+  uint32_t *d_mod, *d_exp, *d_bases, *d_out;
   const size_t mod_b = groups * (size_t)limbs * 4, exp_b = groups * (size_t)exp_limbs * 4, base_b = count * (size_t)limbs * 4;
   cudaError_t e = bufs.alloc(&d_mod, mod_b);
   if (e == cudaSuccess) e = bufs.alloc(&d_exp, exp_b);
   if (e == cudaSuccess) e = bufs.alloc(&d_bases, base_b);
   if (e == cudaSuccess) e = bufs.alloc(&d_out, base_b);
-  if (e == cudaSuccess && !coop) e = bufs.alloc(&d_gc, groups * (size_t)(3 * plan.Lp + plan.K) * 4);
-  if (e == cudaSuccess && !coop) e = bufs.alloc(&d_dig, groups * (size_t)plan.ndigits);
   if (e != cudaSuccess) return fail(DKG_ERR_NOMEM, std::string("grouped cudaMalloc: ") + cudaGetErrorString(e));
   CUDA_TRY(cudaMemcpyAsync(d_mod, moduli, mod_b, cudaMemcpyHostToDevice, d->stream));
   CUDA_TRY(cudaMemcpyAsync(d_exp, exps, exp_b, cudaMemcpyHostToDevice, d->stream));
   CUDA_TRY(cudaMemcpyAsync(d_bases, bases, base_b, cudaMemcpyHostToDevice, d->stream));
-  rc = coop ? launch_coop_grouped_batch(d, cplan, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, per_group, limbs)
-            : launch_grouped(d, plan, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, per_group, limbs, d_gc, d_dig);
+  rc = launch_grouped(d, bufs, moduli, exps, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, per_group, limbs);
   if (rc != DKG_OK) return rc;
   CUDA_TRY(cudaMemcpyAsync(out, d_out, base_b, cudaMemcpyDeviceToHost, d->stream));
   CUDA_TRY(cudaStreamSynchronize(d->stream));
@@ -1514,20 +1342,10 @@ extern "C" int dkg_biprime_v_batch(int device, const uint32_t* moduli, const uin
   int rc = device_state(device, &d);
   if (rc != DKG_OK) return rc;
   CUDA_TRY(cudaSetDevice(device));
-  int ebits = 0;
-  for (size_t g = 0; g < groups; ++g) ebits = std::max(ebits, dkg_host::bit_length(exps + g * (size_t)exp_limbs, exp_limbs));
   const size_t count = groups * (size_t)correct;
   DeviceLease lease(d, d->stream);
-  CoopGroupedPlan cplan;
-  const bool coop = plan_coop_grouped(d, moduli, groups, limbs, ebits, count, &cplan);
-  GroupedPlan plan;
-  if (!coop) {
-    rc = plan_grouped(d, limbs, ebits, count, &plan);
-    if (rc != DKG_OK) return rc;
-  }
   DevBufs bufs(d->stream);
-  uint32_t *d_mod, *d_exp, *d_g, *d_bases, *d_out, *d_gc = nullptr;
-  uint8_t* d_dig = nullptr;
+  uint32_t *d_mod, *d_exp, *d_g, *d_bases, *d_out;
   int8_t* d_sym;
   int *d_pick, *d_count;
   const size_t mod_b = groups * (size_t)limbs * 4, exp_b = groups * (size_t)exp_limbs * 4;
@@ -1537,8 +1355,6 @@ extern "C" int dkg_biprime_v_batch(int device, const uint32_t* moduli, const uin
   if (e == cudaSuccess) e = bufs.alloc(&d_g, g_b);
   if (e == cudaSuccess) e = bufs.alloc(&d_bases, base_b);
   if (e == cudaSuccess) e = bufs.alloc(&d_out, base_b);
-  if (e == cudaSuccess && !coop) e = bufs.alloc(&d_gc, groups * (size_t)(3 * plan.Lp + plan.K) * 4);
-  if (e == cudaSuccess && !coop) e = bufs.alloc(&d_dig, groups * (size_t)plan.ndigits);
   if (e == cudaSuccess) e = bufs.alloc(&d_sym, groups * (size_t)g_per_candidate);
   if (e == cudaSuccess) e = bufs.alloc(&d_pick, count * sizeof(int));
   if (e == cudaSuccess) e = bufs.alloc(&d_count, groups * sizeof(int));
@@ -1553,8 +1369,7 @@ extern "C" int dkg_biprime_v_batch(int device, const uint32_t* moduli, const uin
   dkg::gather_g_kernel<<<gblocks, 256, 0, d->stream>>>(d_g, d_pick, limbs, groups, g_per_candidate, correct, d_bases);
   g_launches.fetch_add(3);
   CUDA_TRY(cudaGetLastError());
-  rc = coop ? launch_coop_grouped_batch(d, cplan, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, correct, limbs)
-            : launch_grouped(d, plan, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, correct, limbs, d_gc, d_dig);
+  rc = launch_grouped(d, bufs, moduli, exps, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, correct, limbs);
   if (rc != DKG_OK) return rc;
   dkg::clear_unused_kernel<<<gblocks, 256, 0, d->stream>>>(d_out, d_count, limbs, groups, correct);
   g_launches.fetch_add(1);
@@ -1672,7 +1487,6 @@ extern "C" int dkg_biprime_verdict(int device, const uint32_t* moduli, const uin
 // the reference's test and benchmark set-up, distributed_keygen.py:203-226) the d+1 partial
 // decryptions and the combination of _decrypt_sequence_raw (:463-466, :510-515) run back to back on
 // the device: the ciphertexts are uploaded once, the partials never visit the host unless asked for.
-#include <thread>
 
 struct dkg_threshold_ctx {
   struct Dev {
@@ -1712,38 +1526,30 @@ int launch_threshold_multi(dkg_threshold_ctx::Dev& dv, int S, const uint32_t* d_
   DeviceState* d = dv.dev;
   CUDA_TRY(cudaSetDevice(d->device));
   const int Lp = c0->nLp, l2 = c0->limbs;
-  const unsigned long long ngroups = (rows + 31) / 32;
   const size_t pair_words = rows * (size_t)(2 * Lp);
   // negative exponents: the party's RESULTS are inverted inside the kernel (pair_invert, exact
-  // per-element status) or, with DKG_INKERNEL_INVERSE=0, by the batched inversion behind it
+  // per-element status, DKG_INKERNEL_INVERSE=1) or by the batched inversion behind it
   const bool inv_in_kernel = c0->nsq_inv;
   unsigned int negative_mask = 0;
-  bool any_neg = false;
+  size_t inv_words = 0, scratch_words = (size_t)c0->ctas * c0->nwarps * dv.multi_scratch_per_warp;
   for (int p = 0; p < S; ++p) {
-    if (dv.parties[p]->negative && inv_in_kernel) negative_mask |= 1u << p;
-    any_neg = any_neg || (dv.parties[p]->negative && !inv_in_kernel);
+    const dkg_modexp_ctx* c = dv.parties[p];
+    if (c->negative && inv_in_kernel) negative_mask |= 1u << p;
+    if (!c->negative || inv_in_kernel) continue;
+    inv_words = batchinv_area(c, rows);   // the same for every party (one N)
+    scratch_words = std::max(scratch_words, (size_t)c->ctas * c->warps * c->scratch_per_warp);   // its direct redo
   }
-  const size_t gwords = (size_t)c0->Lp * 32;
-  const int nchain = inversion_chain_warps(d, c0, ngroups);
-  const int chain_len = (int)((ngroups + nchain - 1) / nchain);
-  const size_t inv_words = any_neg ? 2 * ngroups * gwords + (size_t)nchain * gwords + (size_t)nchain * 32 + 32 * (size_t)S : 0;
-  int rc = ensure_aux(d, (size_t)(S + 1) * pair_words + inv_words);
-  const int total_warps = c0->ctas * c0->nwarps;
-  size_t scratch_words = (size_t)total_warps * dv.multi_scratch_per_warp;
-  if (any_neg) scratch_words = std::max(scratch_words, (size_t)c0->ctas * c0->warps * c0->scratch_per_warp);
+  int rc = ensure_aux(d, inv_words + (size_t)(S + 1) * pair_words);
   if (rc == DKG_OK) rc = ensure_scratch(d, scratch_words);
   if (rc != DKG_OK) return rc;
-  uint32_t* pairs_in = d->aux;
-  uint32_t* pairs_out = d->aux + pair_words;
-  uint32_t* inv_area = pairs_out + (size_t)S * pair_words;
+  uint32_t* pairs_in = d->aux + inv_words;
+  uint32_t* pairs_out = pairs_in + pair_words;
   CUDA_TRY(cudaMemsetAsync(d_st, 0, rows * (size_t)S, stream));
   dkg::NsqIoParams e{};
   e.in = d_bases; e.out = pairs_in; e.count = rows; e.io_limbs = l2; e.Lp = Lp; e.consts = c0->d_nio; e.n0inv = c0->n_n0inv;
   e.mrows = nullptr; e.m_limbs = 0;
   dkg::nsq_entry_kernel<<<(unsigned)((rows + 63) / 64), 64, 0, stream>>>(e);
   CUDA_TRY(cudaMemsetAsync(d->counter, 0, sizeof(unsigned int), stream));
-  int ctas = c0->ctas;
-  if (ngroups < (unsigned long long)total_warps) ctas = (int)((ngroups + c0->nwarps - 1) / c0->nwarps);
   dkg::NsqMultiParams q{};
   q.pairs_in = pairs_in; q.pairs_out = pairs_out; q.count = rows; q.consts = c0->d_nconsts; q.digits = dv.d_digits;
   q.nparties = S; q.nwin = dv.multi_nwin; q.wbits = dv.multi_w; q.scratch = d->scratch;
@@ -1751,7 +1557,7 @@ int launch_threshold_multi(dkg_threshold_ctx::Dev& dv, int S, const uint32_t* d_
   q.scratch_per_warp = dv.multi_scratch_per_warp; q.scratch_q_offset = dv.multi_q_offset; q.counter = d->counter;
   {
     KernelTimer kt(d, stream);
-    dv.multi_kernel<<<ctas, c0->nwarps * 32, c0->nsmem, stream>>>(q);
+    dv.multi_kernel<<<wave_ctas(c0->ctas, c0->nwarps, rows), c0->nwarps * 32, c0->nsmem, stream>>>(q);
   }
   dkg::NsqIoParams x = e;
   x.in = pairs_out; x.out = d_part; x.count = rows * (size_t)S;
@@ -1762,32 +1568,41 @@ int launch_threshold_multi(dkg_threshold_ctx::Dev& dv, int S, const uint32_t* d_
     dkg_modexp_ctx* c = dv.parties[p];
     uint32_t* out_p = d_part + (size_t)p * rows * l2;
     if (c->negative && !inv_in_kernel) {
-      dkg::BatchInvParams b{};
-      b.bases = out_p; b.count = rows; b.in_limbs = l2; b.consts = c->d_consts; b.n0inv = c->n0inv;
-      b.chain_s = inv_area; b.chain_p = inv_area + ngroups * gwords; b.scratch = inv_area + 2 * ngroups * gwords;
-      b.chain_status = b.scratch + (size_t)nchain * gwords;
-      b.any_bad = reinterpret_cast<unsigned int*>(b.chain_status + (size_t)nchain * 32 + 32 * (size_t)p);
-      b.plain_out = out_p;   // in place: a chain warp reads all its groups before it writes any
-      b.nchain_warps = nchain; b.chain_len = chain_len;
-      CUDA_TRY(cudaMemsetAsync(b.any_bad, 0, sizeof(unsigned int), stream));
-      const int blocks = (nchain + c->inv_warps - 1) / c->inv_warps;
-      c->inv_kernel<<<blocks, c->inv_warps * 32, c->inv_smem, stream>>>(b);
-      CUDA_TRY(cudaMemsetAsync(d->counter, 0, sizeof(unsigned int), stream));
-      dkg::ModexpParams m{};
-      m.bases = d_bases; m.out = out_p; m.status = d_st + (size_t)p * rows; m.count = rows; m.in_limbs = l2;
-      m.consts = c->d_consts; m.ops = c->d_ops; m.nops = c->nops; m.tab_entries = c->tab_entries; m.table_odd = c->table_odd;
-      m.negative = 1; m.n0inv = c->n0inv; m.scratch = d->scratch; m.scratch_per_warp = c->scratch_per_warp;
-      m.scratch_q_offset = c->scratch_q_offset; m.counter = d->counter; m.run_if = b.any_bad;
-      int dctas = c->ctas;
-      if (ngroups < (unsigned long long)(c->ctas * c->warps)) dctas = (int)((ngroups + c->warps - 1) / c->warps);
-      c->kernel<<<dctas, c->warps * 32, c->smem, stream>>>(m);
-      CUDA_TRY(cudaGetLastError());
-      g_launches.fetch_add(2);
+      dkg::BatchInvParams inv;
+      rc = launch_batchinv(c, out_p, rows, out_p, stream, &inv);
+      if (rc == DKG_OK) rc = launch_direct(c, d_bases, out_p, d_st + (size_t)p * rows, nullptr, rows, stream, nullptr, inv.any_bad);
+      if (rc != DKG_OK) return rc;
     }
     rc = launch_range_check(c, d_bases, out_p, d_st + (size_t)p * rows, rows, stream);
     if (rc != DKG_OK) return rc;
   }
   return DKG_OK;
+}
+
+// Every party's partial decryption of `rows` ciphertexts on one device, d_part: [S][rows][l2],
+// d_st: [S][rows].  A few ciphertexts: every party's exponentiation in ONE cooperative launch (one
+// warp per (party, ciphertext)); otherwise the shared squaring chain, else one call per party.
+int launch_partials(const dkg_threshold_ctx* t, dkg_threshold_ctx::Dev& dv, const uint32_t* d_in, uint32_t* d_part,
+                    uint8_t* d_st, size_t rows, cudaStream_t s) {
+  const int S = t->shares;
+  bool fused = S <= dkg::kCoopMaxParties;
+  for (int p = 0; p < S; ++p) fused = fused && dv.parties[p]->coop && rows * (size_t)S <= dv.parties[p]->coop_max;
+  int rc = DKG_OK;
+  if (fused) {
+    rc = launch_modexp_coop_parties(dv.parties.data(), S, d_in, d_part, d_st, rows, s, nullptr, 0);
+    for (int p = 0; p < S && rc == DKG_OK; ++p)
+      rc = launch_range_check(dv.parties[p], d_in, d_part + (size_t)p * rows * t->l2, d_st + (size_t)p * rows, rows, s);
+    return rc;
+  }
+  if (dv.multi_kernel != nullptr) {
+    rc = launch_threshold_multi(dv, S, d_in, d_part, d_st, rows, s);
+    if (rc != DKG_ERR_NOMEM) return rc;
+    dv.multi_kernel = nullptr;   // no room for the bucket scratch: one exponentiation per party from here on
+    rc = DKG_OK;
+  }
+  for (int p = 0; p < S && rc == DKG_OK; ++p)
+    rc = launch_modexp(dv.parties[p], d_in, d_part + (size_t)p * rows * t->l2, d_st + (size_t)p * rows, rows, s);
+  return rc;
 }
 
 // what one device does with its shard, chunk by chunk, alternating between its two streams so the
@@ -1864,30 +1679,9 @@ int run_threshold_shard(dkg_threshold_ctx* t, dkg_threshold_ctx::Dev& dv, const 
     {
       DeviceLease lease(dv.dev, s);
       if (job.mode == 1) {
-        rc = launch_modexp(dv.parties[job.party], B.in, B.part, B.st, nullptr, rows, s);
+        rc = launch_modexp(dv.parties[job.party], B.in, B.part, B.st, rows, s);
       } else {
-        if (job.mode == 0 || job.mode == 3) {
-          // a few ciphertexts: every party's exponentiation in ONE cooperative launch (one warp per
-          // (party, ciphertext)); otherwise one wave launch per party
-          bool fused = S <= dkg::kCoopMaxParties;
-          for (int p = 0; p < S; ++p) fused = fused && dv.parties[p]->coop && dv.parties[p]->use_nsq && rows * (size_t)S <= dv.parties[p]->coop_max;
-          if (!fused && dv.multi_kernel != nullptr) {
-            rc = launch_threshold_multi(dv, S, B.in, B.part, B.st, rows, s);
-            if (rc == DKG_ERR_NOMEM) {   // no room for the bucket scratch: one exponentiation per party from here on
-              dv.multi_kernel = nullptr;
-              rc = DKG_OK;
-              for (int p = 0; p < S && rc == DKG_OK; ++p)
-                rc = launch_modexp(dv.parties[p], B.in, B.part + (size_t)p * rows * l2, B.st + (size_t)p * rows, nullptr, rows, s);
-            }
-          } else if (fused) {
-            rc = launch_modexp_coop_parties(dv.parties.data(), S, B.in, B.part, B.st, rows, s, nullptr, 0);
-            for (int p = 0; p < S && rc == DKG_OK; ++p)
-              rc = launch_range_check(dv.parties[p], B.in, B.part + (size_t)p * rows * l2, B.st + (size_t)p * rows, rows, s);
-          } else {
-            for (int p = 0; p < S && rc == DKG_OK; ++p)
-              rc = launch_modexp(dv.parties[p], B.in, B.part + (size_t)p * rows * l2, B.st + (size_t)p * rows, nullptr, rows, s);
-          }
-        }
+        if (job.mode == 0 || job.mode == 3) rc = launch_partials(t, dv, B.in, B.part, B.st, rows, s);
         if (rc == DKG_OK && job.mode != 3) rc = launch_combine(dv.combine, B.part, B.out, B.st + (size_t)S * rows, rows, s);
       }
       if (rc != DKG_OK) { *err = g_err; break; }
@@ -1942,11 +1736,12 @@ int setup_threshold_multi(dkg_threshold_ctx::Dev& dv, int shares, const uint32_t
   int ebits = 1;
   for (int p = 0; p < shares; ++p) {
     const dkg_modexp_ctx* c = dv.parties[p];
-    if (!c->nsq || !c->use_nsq || c->ct_table || c->nshape.K != c0->nshape.K || c->nshape.M != c0->nshape.M || c->nsq_bg != c0->nsq_bg) return DKG_OK;
+    if (!c->nsq || c->ct_table || c->nshape.K != c0->nshape.K || c->nshape.M != c0->nshape.M || c->nsq_bg != c0->nsq_bg) return DKG_OK;
     if (c->negative && c->inv_kernel == nullptr) return DKG_OK;
     ebits = std::max(ebits, c->ebits);
   }
-  dkg::NsqMultiFn kernel = lookup_nsq_multi(c0->nshape.K, c0->nshape.M, c0->nsq_bg);
+  const dkg::ShapeKernels kernels = lookup_kernels(c0->nshape.K, c0->nshape.M);
+  const dkg::NsqMultiFn kernel = c0->nsq_bg ? kernels.multi_bg : kernels.multi;
   if (!kernel) return DKG_OK;
   const size_t slot_words = (size_t)2 * c0->nLs * 32;   // one pair in lane layout
   const size_t total_warps = (size_t)c0->ctas * c0->nwarps;
@@ -2071,25 +1866,7 @@ int dkg_threshold_decrypt_batch_device(dkg_threshold_ctx* t, const uint32_t* d_c
   cudaStream_t s = (cudaStream_t)stream;
   const int S = t->shares;
   DeviceLease lease(dv.dev, s);
-  bool fused = S <= dkg::kCoopMaxParties;
-  for (int p = 0; p < S; ++p) fused = fused && dv.parties[p]->coop && dv.parties[p]->use_nsq && count * (size_t)S <= dv.parties[p]->coop_max;
-  int rc = DKG_OK;
-  if (!fused && dv.multi_kernel != nullptr) {
-    rc = launch_threshold_multi(dv, S, d_ciphertexts, d_partials, d_status, count, s);
-    if (rc == DKG_ERR_NOMEM) {   // no room for the bucket scratch: one exponentiation per party from here on
-      dv.multi_kernel = nullptr;
-      rc = DKG_OK;
-      for (int p = 0; p < S && rc == DKG_OK; ++p)
-        rc = launch_modexp(dv.parties[p], d_ciphertexts, d_partials + (size_t)p * count * t->l2, d_status + (size_t)p * count, nullptr, count, s);
-    }
-  } else if (fused) {
-    rc = launch_modexp_coop_parties(dv.parties.data(), S, d_ciphertexts, d_partials, d_status, count, s, nullptr, 0);
-    for (int p = 0; p < S && rc == DKG_OK; ++p)
-      rc = launch_range_check(dv.parties[p], d_ciphertexts, d_partials + (size_t)p * count * t->l2, d_status + (size_t)p * count, count, s);
-  } else {
-    for (int p = 0; p < S && rc == DKG_OK; ++p)
-      rc = launch_modexp(dv.parties[p], d_ciphertexts, d_partials + (size_t)p * count * t->l2, d_status + (size_t)p * count, nullptr, count, s);
-  }
+  int rc = launch_partials(t, dv, d_ciphertexts, d_partials, d_status, count, s);
   if (rc == DKG_OK) rc = launch_combine(dv.combine, d_partials, d_plaintexts, d_status + (size_t)S * count, count, s);
   return rc;
 }

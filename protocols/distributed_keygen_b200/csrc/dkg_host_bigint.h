@@ -55,6 +55,35 @@ inline Limbs pow2_mod(size_t bits, const Limbs& n) {
   return x;
 }
 
+// -a mod 2^(32 a.size())
+inline Limbs negate(const Limbs& a) {
+  Limbs r(a.size());
+  uint64_t carry = 1;
+  for (size_t i = 0; i < a.size(); ++i) {
+    uint64_t t = (uint64_t)(~a[i]) + carry;
+    r[i] = (uint32_t)t;
+    carry = t >> 32;
+  }
+  return r;
+}
+
+// a^2 by schoolbook, without leading zero limbs (at least one limb)
+inline Limbs square(const Limbs& a) {
+  const size_t n = a.size();
+  Limbs r(2 * n, 0);
+  for (size_t i = 0; i < n; ++i) {
+    uint64_t carry = 0;
+    for (size_t j = 0; j < n; ++j) {
+      uint64_t t = (uint64_t)a[i] * a[j] + r[i + j] + carry;
+      r[i + j] = (uint32_t)t;
+      carry = t >> 32;
+    }
+    r[i + n] = (uint32_t)carry;
+  }
+  while (r.size() > 1 && r.back() == 0) r.pop_back();
+  return r;
+}
+
 // -n^-1 mod 2^(32*K) for odd n (Hensel lifting, one limb at a time)
 inline Limbs neg_inv_block(const Limbs& n, int K) {
   // 32-bit inverse of n[0] by Newton
@@ -75,14 +104,7 @@ inline Limbs neg_inv_block(const Limbs& n, int K) {
       carry = t >> 32;
     }
   }
-  // negate mod 2^(32K)
-  uint64_t carry = 1;
-  for (int i = 0; i < K; ++i) {
-    uint64_t t = (uint64_t)(~inv[i]) + carry;
-    inv[i] = (uint32_t)t;
-    carry = t >> 32;
-  }
-  return inv;
+  return negate(inv);
 }
 
 // (a + b) mod n and (a - b) mod n for a, b < n (same length)
