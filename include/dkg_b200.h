@@ -78,7 +78,15 @@ unsigned long long dkg_launch_count(void);
  *                      (distributed_keygen.py:314-382); 0 disables it.  Environment: DKG_COOP_MAX,
  *                      DKG_COOP=0.
  *   "coop_grouped_max" same for the grouped (biprimality) entry points, per call.  Environment:
- *                      DKG_COOP_GROUPED_MAX. */
+ *                      DKG_COOP_GROUPED_MAX.
+ *   "ct_table"         1: constant-time table access -- every window multiplication reads the
+ *                      whole window table (and the Montgomery one) under a mask, so no memory
+ *                      address and no branch depends on a digit of the exponent (DESIGN.md §2.11).
+ *                      A fixed-exponent context (dkg_modexp_ctx_create, the threshold context)
+ *                      takes the setting when it is created; dkg_modexp_grouped and
+ *                      dkg_biprime_v_batch read it on every call.  Default 0.  Environment:
+ *                      DKG_CT_TABLE=1.
+ *   "time_kernels"     see dkg_kernel_times below. */
 int dkg_config_set(const char* key, long value);
 int dkg_config_get(const char* key, long* value);
 /* With dkg_config_set("time_kernels", 1) every launch of an exponentiation kernel of the pair

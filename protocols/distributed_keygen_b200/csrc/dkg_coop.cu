@@ -16,9 +16,9 @@ static cudaError_t launch_nsq_t(const CoopNsqParams& p, int ctas, int warps, siz
   kernel<<<ctas, warps * 32, smem, stream>>>(p);
   return cudaGetLastError();
 }
-template <int K, int THREADS>
+template <int K, int THREADS, bool CT>
 static cudaError_t launch_grouped_t(const CoopGroupedParams& p, int ctas, int warps, size_t smem, cudaStream_t stream) {
-  auto kernel = coop_grouped_kernel<K, THREADS>;
+  auto kernel = coop_grouped_kernel<K, THREADS, CT>;
   cudaError_t e = cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return e;
   kernel<<<ctas, warps * 32, smem, stream>>>(p);
@@ -44,9 +44,12 @@ cudaError_t launch_coop_nsq(int K, const CoopNsqParams& p, int ctas, int warps, 
   if (K == 12) return launch_nsq_t<12, 256>(p, ctas, warps, smem, stream);
   return cudaErrorInvalidValue;
 }
-cudaError_t launch_coop_grouped(int K, const CoopGroupedParams& p, int ctas, int warps, size_t smem, cudaStream_t stream) {
-  if (K == 6) return launch_grouped_t<6, 512>(p, ctas, warps, smem, stream);
-  if (K == 12) return launch_grouped_t<12, 256>(p, ctas, warps, smem, stream);
+cudaError_t launch_coop_grouped(int K, bool ct_table, const CoopGroupedParams& p, int ctas, int warps, size_t smem,
+                                cudaStream_t stream) {
+  if (K == 6) return ct_table ? launch_grouped_t<6, 512, true>(p, ctas, warps, smem, stream)
+                              : launch_grouped_t<6, 512, false>(p, ctas, warps, smem, stream);
+  if (K == 12) return ct_table ? launch_grouped_t<12, 256, true>(p, ctas, warps, smem, stream)
+                               : launch_grouped_t<12, 256, false>(p, ctas, warps, smem, stream);
   return cudaErrorInvalidValue;
 }
 

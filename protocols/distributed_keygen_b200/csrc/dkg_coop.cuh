@@ -760,7 +760,8 @@ __global__ void __launch_bounds__(THREADS) coop_combine_kernel(const CoopCombine
 }
 
 // ---- grouped exponentiation (per-instance modulus and exponent), one instance per warp ---------------
-template <int K, int THREADS>
+// CT: constant-time table access (DESIGN.md §2.11), its own instantiation chosen by the host
+template <int K, int THREADS, bool CT = false>
 __global__ void __launch_bounds__(THREADS) coop_grouped_kernel(const CoopGroupedParams p) {
   using namespace coop;
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -868,25 +869,50 @@ __global__ void __launch_bounds__(THREADS) coop_grouped_kernel(const CoopGrouped
     }
     __syncwarp();
     const uint32_t* ex = p.exps + g * (unsigned long long)p.exp_limbs;
-    auto digit = [&](int tdig) -> uint32_t {
-      const int lowbit = p.wbits * (p.ndigits - 1 - tdig);
-      uint32_t v = 0;
-      for (int bb = 0; bb < p.wbits; ++bb) {
-        const int bit = lowbit + bb;
-        if (bit < 32 * p.exp_limbs && ((ex[bit / 32] >> (bit % 32)) & 1u)) v |= 1u << bb;
+    if constexpr (CT) {
+      // constant-time table access: from ONE, every window scans all entries and ONE (digit 0)
+      // under a mask into Y, lane-strided as in coop_nsq_kernel, and multiplies by Y; the digit
+      // comes from shifts and masks (the conditions are on bit positions only)
+      auto digit = [&](int tdig) -> uint32_t {
+        const int lowbit = p.wbits * (p.ndigits - 1 - tdig);
+        const int wi = lowbit / 32;
+        const uint64_t lo = wi < p.exp_limbs ? ex[wi] : 0u, hi = wi + 1 < p.exp_limbs ? ex[wi + 1] : 0u;
+        return (uint32_t)((hi << 32 | lo) >> (lowbit % 32)) & ((1u << p.wbits) - 1u);
+      };
+      copy(X, ONE, Lc);
+      for (int td = 0; td < p.ndigits; ++td) {
+        if (td > 0)
+          for (int q = 0; q < p.wbits; ++q) montmul<K>(w, sX, sX, sX, 0, 0);
+        const uint32_t dg = digit(td), di = dg - 1u, m0 = 0u - (uint32_t)(dg == 0u);
+        for (int l = lane; l < Lc; l += 32) {
+          uint32_t acc = ONE[l] & m0;
+          for (int k = 0; k < tn; ++k) acc |= tab[(size_t)k * Lc + l] & (0u - (uint32_t)((uint32_t)k == di));
+          Y[l] = acc;
+        }
+        __syncwarp();
+        montmul<K>(w, sX, sX, sY, 0, 0);
       }
-      return v;
-    };
-    {
-      const uint32_t d0 = digit(0);
-      if (d0) copy(X, tab + (size_t)(d0 - 1) * Lc, Lc); else copy(X, ONE, Lc);
-      __syncwarp();
-    }
-    for (int td = 1; td < p.ndigits; ++td) {
-      for (int q = 0; q < p.wbits; ++q) montmul<K>(w, sX, sX, sX, 0, 0);
-      const uint32_t dg = digit(td);
-      if (dg) { copy(Y, tab + (size_t)(dg - 1) * Lc, Lc); __syncwarp(); montmul<K>(w, sX, sX, sY, 0, 0); }
-      else montmul<K>(w, sX, sX, sONE, 0, 0);
+    } else {
+      auto digit = [&](int tdig) -> uint32_t {
+        const int lowbit = p.wbits * (p.ndigits - 1 - tdig);
+        uint32_t v = 0;
+        for (int bb = 0; bb < p.wbits; ++bb) {
+          const int bit = lowbit + bb;
+          if (bit < 32 * p.exp_limbs && ((ex[bit / 32] >> (bit % 32)) & 1u)) v |= 1u << bb;
+        }
+        return v;
+      };
+      {
+        const uint32_t d0 = digit(0);
+        if (d0) copy(X, tab + (size_t)(d0 - 1) * Lc, Lc); else copy(X, ONE, Lc);
+        __syncwarp();
+      }
+      for (int td = 1; td < p.ndigits; ++td) {
+        for (int q = 0; q < p.wbits; ++q) montmul<K>(w, sX, sX, sX, 0, 0);
+        const uint32_t dg = digit(td);
+        if (dg) { copy(Y, tab + (size_t)(dg - 1) * Lc, Lc); __syncwarp(); montmul<K>(w, sX, sX, sY, 0, 0); }
+        else montmul<K>(w, sX, sX, sONE, 0, 0);
+      }
     }
     // ---- out of the Montgomery domain, canonical residue
     {

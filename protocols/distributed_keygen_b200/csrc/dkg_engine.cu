@@ -60,11 +60,12 @@ void append_lane_replicated(std::vector<uint32_t>& out, const std::vector<uint32
 }
 }  // namespace
 namespace dkg {
-void launch_group_setup(const GroupedParams& p, cudaStream_t stream);
+void launch_group_setup(const GroupedParams& p, bool ct_table, cudaStream_t stream);
 // dkg_coop.cu: the cooperative (warp-per-operand) latency kernels
 int coop_max_warps(int K, bool pair_kernel);
 cudaError_t launch_coop_nsq(int K, const CoopNsqParams& p, int ctas, int warps, size_t smem, cudaStream_t stream);
-cudaError_t launch_coop_grouped(int K, const CoopGroupedParams& p, int ctas, int warps, size_t smem, cudaStream_t stream);
+cudaError_t launch_coop_grouped(int K, bool ct_table, const CoopGroupedParams& p, int ctas, int warps, size_t smem,
+                                cudaStream_t stream);
 cudaError_t launch_coop_combine(int K, const CoopCombineParams& p, int ctas, int warps, size_t smem, cudaStream_t stream);
 }  // namespace dkg
 namespace {
@@ -727,7 +728,8 @@ int dkg_modexp_ctx_create(int device, const uint32_t* modulus, int mod_limbs, co
   ctx->Lp = shape.K * shape.M;
   ctx->negative = exp_negative ? 1 : 0;
   const dkg::ShapeKernels kernels = lookup_kernels(shape.K, shape.M);
-  ctx->kernel = kernels.fixed;
+  ctx->ct_table = ct_table_setting();
+  ctx->kernel = ctx->ct_table ? kernels.fixed_ct : kernels.fixed;
   if (!ctx->kernel) { delete ctx; return fail(DKG_ERR_UNSUPPORTED, "kernel shape not compiled"); }
 
   const int Lp = ctx->Lp, K = shape.K;
@@ -754,7 +756,6 @@ int dkg_modexp_ctx_create(int device, const uint32_t* modulus, int mod_limbs, co
   // windows (DKG_SLIDING_WINDOW=1) save 23 % of the multiplications (~1.5 % of the run time in the
   // pair arithmetic) at the price of an exponent-dependent operation list, as in mpz_powm.
   std::vector<uint32_t> ops;
-  ctx->ct_table = ct_table_setting();
   if (const char* sw = getenv("DKG_SLIDING_WINDOW"); sw && atoi(sw) != 0 && !ctx->ct_table) {
     ctx->wbits = choose_window(ctx->ebits, 7, sliding_window_cost);
     ops = sliding_window_ops(exponent, ctx->ebits, ctx->wbits, &ctx->tab_entries, &ctx->nmul);
@@ -1178,9 +1179,10 @@ struct GroupedPlan {
   dkg::GroupedFn kernel = nullptr;
   int Lp = 0, K = 0, Ka = 0, wbits = 1, ndigits = 1, warps = 1, ctas = 1;   // K, Lp: slot layout; Ka: arithmetic block
   size_t smem = 0, q_off = 0, scratch_per_warp = 0;
+  bool ct_table = false;   // constant-time table access: narrower windows, one more table slot
 };
 
-int plan_grouped(DeviceState* d, int limbs, int ebits, size_t count, GroupedPlan* plan) {
+int plan_grouped(DeviceState* d, int limbs, int ebits, size_t count, bool ct_table, GroupedPlan* plan) {
   if (const char* f = getenv("DKG_GROUPED_SHAPE")) {  // tuning knob: "K,M"
     int k = 0, m = 0;
     if (sscanf(f, "%d,%d", &k, &m) == 2 && k * m >= limbs && (plan->kernel = lookup_kernels(k, m).grouped) != nullptr) plan->shape = Shape{k, m};
@@ -1201,14 +1203,16 @@ int plan_grouped(DeviceState* d, int limbs, int ebits, size_t count, GroupedPlan
   plan->Ka = plan->shape.K;
   plan->K = plan->shape.K + (plan->shape.K & 1);
   plan->Lp = plan->K * plan->shape.M;
-  plan->wbits = choose_window(ebits, 6, fixed_window_cost);
+  plan->ct_table = ct_table;
+  if (ct_table) plan->kernel = lookup_kernels(plan->shape.K, plan->shape.M).grouped_ct;   // (compiled with .grouped)
+  plan->wbits = choose_window(ebits, 6, ct_table ? ct_window_cost : fixed_window_cost);
   plan->ndigits = std::max(1, (ebits + plan->wbits - 1) / plan->wbits);
   const size_t per_warp_smem = ((size_t)2 * plan->Lp + plan->K) * 32 * 4;
   const size_t sched_bytes = (((size_t)dkg::sched_total_words_closed(plan->shape.M) * 4 + 15) / 16) * 16;
   plan->warps = (int)std::min<size_t>(DKG_MAX_THREADS / 32, (kMaxDynSmem - sched_bytes) / per_warp_smem);
   if (plan->warps < 1) return fail(DKG_ERR_UNSUPPORTED, "operand too wide for shared memory");
   plan->smem = sched_bytes + per_warp_smem * plan->warps;
-  const size_t tsize = ((size_t)1 << plan->wbits) - 1;
+  const size_t tsize = ((size_t)1 << plan->wbits) - 1 + (ct_table ? 1 : 0);   // (+ the slot ct_select writes)
   plan->q_off = std::max<size_t>(tsize, 1) * (size_t)plan->Lp * 32;
   plan->scratch_per_warp = plan->q_off + (size_t)3 * plan->Lp * 32;  // Q | R2 | ONER in lane layout
   plan->ctas = wave_ctas(d->sm_count, plan->warps, count);
@@ -1225,18 +1229,20 @@ struct CoopGroupedPlan {
   int K = 0, nb = 0, Lc = 0, wbits = 1, ndigits = 1, ctas = 1, warps = 1;
   size_t smem = 0, per_warp = 0;
   dkg::CoopPlanTable full{}, low{};
+  bool ct_table = false;   // constant-time table access (the selection goes to Y: no extra slot)
 };
 
 // true if this batch should take the cooperative kernel (moduli: host copy, for the widest one)
 bool plan_coop_grouped(DeviceState* d, const uint32_t* moduli, size_t groups, int limbs, int ebits, size_t count,
-                       CoopGroupedPlan* plan) {
+                       bool ct_table, CoopGroupedPlan* plan) {
   if (count == 0 || count > coop_limit(g_coop_grouped_max, "DKG_COOP_GROUPED_MAX", kCoopGroupedMaxDefault)) return false;
   int maxbits = 1;
   for (size_t g = 0; g < groups; ++g) maxbits = std::max(maxbits, dkg_host::bit_length(moduli + g * (size_t)limbs, limbs));
   const int need = (maxbits + 2 + 31) / 32;   // R >= 4N
   if (!coop_shape(need, &plan->K, &plan->nb)) return false;
   plan->Lc = plan->K * plan->nb;
-  plan->wbits = choose_window(ebits, 6, fixed_window_cost);
+  plan->ct_table = ct_table;
+  plan->wbits = choose_window(ebits, 6, ct_table ? ct_window_cost : fixed_window_cost);
   plan->ndigits = std::max(1, (ebits + plan->wbits - 1) / plan->wbits);
   coop_grid(d, plan->K, false, count, &plan->ctas, &plan->warps);
   plan->smem = (size_t)9 * plan->warps * plan->Lc * 4;
@@ -1255,7 +1261,7 @@ int launch_coop_grouped_batch(DeviceState* d, const CoopGroupedPlan& plan, const
   p.moduli = d_mod; p.exps = d_exp; p.bases = d_bases; p.out = d_out; p.groups = groups; p.per_group = per_group;
   p.limbs = limbs; p.exp_limbs = exp_limbs; p.nb = plan.nb; p.wbits = plan.wbits; p.ndigits = plan.ndigits;
   p.scratch = d->scratch; p.scratch_per_warp = plan.per_warp; p.counter = d->counter; p.full = plan.full; p.low = plan.low;
-  CUDA_TRY(dkg::launch_coop_grouped(plan.K, p, plan.ctas, plan.warps, plan.smem, d->stream));
+  CUDA_TRY(dkg::launch_coop_grouped(plan.K, plan.ct_table, p, plan.ctas, plan.warps, plan.smem, d->stream));
   g_launches.fetch_add(1);
   return DKG_OK;
 }
@@ -1263,17 +1269,19 @@ int launch_coop_grouped_batch(DeviceState* d, const CoopGroupedPlan& plan, const
 // Grouped modexp of groups x per_group device rows on d->stream: the cooperative kernel for small
 // batches, else group setup + wave kernel with per-group constants and digits allocated in `bufs`.
 // moduli, exps: host copies (the plans size themselves for the widest modulus and exponent).
+// The constant-time setting ("ct_table") is read on every call.
 int launch_grouped(DeviceState* d, DevBufs& bufs, const uint32_t* moduli, const uint32_t* exps, const uint32_t* d_mod,
                    const uint32_t* d_exp, int exp_limbs, const uint32_t* d_bases, uint32_t* d_out, size_t groups,
                    int per_group, int limbs) {
   int ebits = 0;
   for (size_t g = 0; g < groups; ++g) ebits = std::max(ebits, dkg_host::bit_length(exps + g * (size_t)exp_limbs, exp_limbs));
   const size_t count = groups * (size_t)per_group;
+  const bool ct_table = ct_table_setting();
   CoopGroupedPlan cplan;
-  if (plan_coop_grouped(d, moduli, groups, limbs, ebits, count, &cplan))
+  if (plan_coop_grouped(d, moduli, groups, limbs, ebits, count, ct_table, &cplan))
     return launch_coop_grouped_batch(d, cplan, d_mod, d_exp, exp_limbs, d_bases, d_out, groups, per_group, limbs);
   GroupedPlan plan;
-  int rc = plan_grouped(d, limbs, ebits, count, &plan);
+  int rc = plan_grouped(d, limbs, ebits, count, ct_table, &plan);
   if (rc != DKG_OK) return rc;
   uint32_t* d_gc;
   uint8_t* d_dig;
@@ -1286,7 +1294,7 @@ int launch_grouped(DeviceState* d, DevBufs& bufs, const uint32_t* moduli, const 
   p.per_group = per_group; p.limbs = limbs; p.exp_limbs = exp_limbs; p.K = plan.K; p.Lp = plan.Lp; p.Ka = plan.Ka;
   p.wbits = plan.wbits; p.ndigits = plan.ndigits; p.gconsts = d_gc; p.digits = d_dig; p.scratch = d->scratch;
   p.scratch_per_warp = plan.scratch_per_warp; p.scratch_q_offset = plan.q_off; p.counter = d->counter;
-  dkg::launch_group_setup(p, d->stream);
+  dkg::launch_group_setup(p, plan.ct_table, d->stream);
   plan.kernel<<<plan.ctas, plan.warps * 32, plan.smem, d->stream>>>(p);
   g_launches.fetch_add(2);
   CUDA_TRY(cudaGetLastError());

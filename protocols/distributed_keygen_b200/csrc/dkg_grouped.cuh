@@ -15,8 +15,10 @@
 
 namespace dkg {
 
-// One thread per group: Montgomery constants and window digits.
-static __global__ void __launch_bounds__(64) group_setup_kernel(const GroupedParams p) {
+// One thread per group: Montgomery constants and window digits (CT: extracted without a branch on
+// the exponent's bits, for the constant-time instantiation of the grouped kernel).
+template <bool CT>
+__global__ void __launch_bounds__(64) group_setup_kernel(const GroupedParams p) {
   const unsigned long long g = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (g >= p.groups) return;
   // arithmetic: blocks of K limbs, Lp limbs per number, R = 2^(32 Lp); memory: slots of KP limbs
@@ -84,16 +86,24 @@ static __global__ void __launch_bounds__(64) group_setup_kernel(const GroupedPar
   uint8_t* dg = p.digits + g * (unsigned long long)p.ndigits;
   for (int t = 0; t < p.ndigits; ++t) {
     const int lowbit = p.wbits * (p.ndigits - 1 - t);
-    unsigned v = 0;
-    for (int b = 0; b < p.wbits; ++b) {
-      const int bit = lowbit + b;
-      if (bit < 32 * p.exp_limbs && ((e[bit / 32] >> (bit % 32)) & 1u)) v |= 1u << b;
+    if constexpr (CT) {
+      // shifts and masks: the only conditions are on bit positions, never on the exponent's bits
+      const int wi = lowbit / 32;
+      const uint64_t lo = wi < p.exp_limbs ? e[wi] : 0u, hi = wi + 1 < p.exp_limbs ? e[wi + 1] : 0u;
+      dg[t] = (uint8_t)(((hi << 32 | lo) >> (lowbit % 32)) & ((1u << p.wbits) - 1u));
+    } else {
+      unsigned v = 0;
+      for (int b = 0; b < p.wbits; ++b) {
+        const int bit = lowbit + b;
+        if (bit < 32 * p.exp_limbs && ((e[bit / 32] >> (bit % 32)) & 1u)) v |= 1u << b;
+      }
+      dg[t] = (uint8_t)v;
     }
-    dg[t] = (uint8_t)v;
   }
 }
 
-template <int K, int M>
+// CT: constant-time table access (DESIGN.md §2.11), its own instantiation chosen by the host
+template <int K, int M, bool CT = false>
 __global__ void __launch_bounds__(DKG_MAX_THREADS, 1) modexp_grouped_kernel(const GroupedParams p) {
   constexpr int KP = kpad<K>;          // slot of one block in memory (odd K: one zero pad limb)
   using V = typename VecSel<KP>::T;
@@ -178,12 +188,26 @@ __global__ void __launch_bounds__(DKG_MAX_THREADS, 1) modexp_grouped_kernel(cons
     }
     for (int v = 0; v < LV; ++v) Xw[v * 32 + lane] = ONEl[(size_t)v * 32 + lane];
     const uint8_t* dg = p.digits + gid * (unsigned long long)p.ndigits;
-    for (int t = 0; t < p.ndigits; ++t) {
-      if (t > 0)
-        for (int s = 0; s < p.wbits; ++s) mont_call<K, M, MONT_SQR, true, true>(io);
-      const int d = dg[t];
-      io.Y = (d == 0) ? (ONEl + lane) : (tab + (size_t)(d - 1) * LV * 32 + lane);
-      mont_call<K, M, MONT_MUL, true, true>(io);
+    if constexpr (CT) {
+      // constant-time table access: every window's multiplier goes through ct_select into the
+      // spare slot after the table, and io.Y stays there; digit 0 (index d - 1 wrapped around)
+      // selects the lane's ONEl
+      V* slot = tab + (size_t)tsize * LV * 32 + lane;
+      io.Y = slot;
+      for (int t = 0; t < p.ndigits; ++t) {
+        if (t > 0)
+          for (int s = 0; s < p.wbits; ++s) mont_call<K, M, MONT_SQR, true, true>(io);
+        ct_select_lane<V, VW>(tab + lane, ONEl + lane, slot, tsize, LV, (uint32_t)dg[t] - 1u);
+        mont_call<K, M, MONT_MUL, true, true>(io);
+      }
+    } else {
+      for (int t = 0; t < p.ndigits; ++t) {
+        if (t > 0)
+          for (int s = 0; s < p.wbits; ++s) mont_call<K, M, MONT_SQR, true, true>(io);
+        const int d = dg[t];
+        io.Y = (d == 0) ? (ONEl + lane) : (tab + (size_t)(d - 1) * LV * 32 + lane);
+        mont_call<K, M, MONT_MUL, true, true>(io);
+      }
     }
     mont_call<K, M, MONT_REDC, true, true>(io);
     canonicalize<K, M>(io, 1);

@@ -13,12 +13,13 @@ using NsqFn = void (*)(const NsqParams);
 using NsqMultiFn = void (*)(const NsqMultiParams);
 using GroupedFn = void (*)(const GroupedParams);
 
+// (_ct: the constant-time table access instantiation, DESIGN.md §2.11)
 struct ShapeKernels {
-  KernelFn fixed = nullptr;        // modexp_fixed_kernel (direct)
+  KernelFn fixed = nullptr, fixed_ct = nullptr;        // modexp_fixed_kernel (direct)
   BatchInvFn batchinv = nullptr;
   NsqFn nsq = nullptr, nsq_bg = nullptr;            // pair arithmetic; _bg: b component in global scratch
   NsqMultiFn multi = nullptr, multi_bg = nullptr;   // shared squaring chain
-  GroupedFn grouped = nullptr;
+  GroupedFn grouped = nullptr, grouped_ct = nullptr;
 };
 
 void find_kernels_group0(int K, int M, ShapeKernels* k);

@@ -6,8 +6,9 @@
 #include "dkg_kernels.inc"
 
 namespace dkg {
-void launch_group_setup(const GroupedParams& p, cudaStream_t stream) {
+void launch_group_setup(const GroupedParams& p, bool ct_table, cudaStream_t stream) {
   const unsigned blocks = (unsigned)((p.groups + 63) / 64);
-  group_setup_kernel<<<blocks, 64, 0, stream>>>(p);
+  if (ct_table) group_setup_kernel<true><<<blocks, 64, 0, stream>>>(p);
+  else group_setup_kernel<false><<<blocks, 64, 0, stream>>>(p);
 }
 }  // namespace dkg

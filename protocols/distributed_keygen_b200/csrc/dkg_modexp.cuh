@@ -14,6 +14,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include "dkg_mont.cuh"
+#include "dkg_ct_select.cuh"
 #include "dkg_modexp_params.h"
 
 namespace dkg {
@@ -336,7 +337,28 @@ __device__ __forceinline__ void fill_schedule(uint32_t* tab) {
   for (int i = threadIdx.x; i < n; i += blockDim.x) tab[i] = sched_entry<M>(i);
 }
 
-template <int K, int M>
+// ct_select accessor for one lane of a warp's window table (vector-major / lane-minor, global
+// memory; every pointer already offset by the lane): entry k, vector v at tab[(k * nvec + v) * 32]
+template <class V, int VW>
+struct LaneTable {
+  const V* tab;
+  const V* onev;   // the Montgomery one, same vector stride
+  V* slot;         // the spare slot the selection goes to
+  int nvec;
+  __device__ __forceinline__ void one(int v, uint32_t (&r)[VW]) const { unpack(onev[(size_t)v * 32], r); }
+  __device__ __forceinline__ void entry(int k, int v, uint32_t (&r)[VW]) const { unpack(tab[((size_t)k * nvec + v) * 32], r); }
+  __device__ __forceinline__ void put(int v, const uint32_t (&r)[VW]) const { V x; pack(x, r); slot[(size_t)v * 32] = x; }
+};
+// Out of line: inlined, the scan's loads and masks raise the register demand of the whole kernel
+// (and the spills of the widest shapes) at a point where most of its state is live.
+template <class V, int VW>
+__device__ __noinline__ void ct_select_lane(const V* tab, const V* onev, V* slot, int n, int nvec, uint32_t idx) {
+  ct_select<VW>(LaneTable<V, VW>{tab, onev, slot, nvec}, n, nvec, idx);
+}
+
+// CT: constant-time table access (DESIGN.md §2.11), its own instantiation chosen by the host, so
+// that the default one is not touched by it
+template <int K, int M, bool CT = false>
 __global__ void __launch_bounds__(DKG_MAX_THREADS, 1) modexp_fixed_kernel(const ModexpParams p) {
   using V = typename VecSel<K>::T;
   constexpr int VW = VecSel<K>::VW;
@@ -436,17 +458,33 @@ __global__ void __launch_bounds__(DKG_MAX_THREADS, 1) modexp_fixed_kernel(const 
         }
       }
       // ---- left to right through the operation list (one list for the whole batch) -------------
-      {
-        const V* src = tab + (size_t)(p.ops[0] & 0xffu) * LV * 32 + lane;
-        for (int v = 0; v < LV; ++v) Xw[v * 32 + lane] = src[(size_t)v * 32];
-      }
-      for (int t = 1; t < p.nops; ++t) {
-        const uint32_t op = p.ops[t];
-        for (uint32_t s = op >> 8; s > 0; --s) mont_call<K, M, MONT_SQR>(io);
-        const uint32_t idx = op & 0xffu;
-        if (idx != 0xffu) {
-          io.Y = idx == 0xfeu ? ONErep : tab + (size_t)idx * LV * 32 + lane;
+      if constexpr (CT) {
+        // constant-time table access (fixed windows only): the first value and every multiplier
+        // come from ct_select into the spare slot after the table, so no address depends on a
+        // digit (dkg_ct_select.cuh); io.Y stays on the slot
+        V* slot = tab + (size_t)tn * LV * 32 + lane;
+        ct_select_lane<V, VW>(tab + lane, ONErep, slot, tn, LV, p.ops[0] & 0xffu);
+        for (int v = 0; v < LV; ++v) Xw[v * 32 + lane] = slot[(size_t)v * 32];
+        io.Y = slot;
+        for (int t = 1; t < p.nops; ++t) {
+          const uint32_t op = p.ops[t];
+          for (uint32_t s = op >> 8; s > 0; --s) mont_call<K, M, MONT_SQR>(io);
+          ct_select_lane<V, VW>(tab + lane, ONErep, slot, tn, LV, op & 0xffu);
           mont_call<K, M, MONT_MUL>(io);
+        }
+      } else {
+        {
+          const V* src = tab + (size_t)(p.ops[0] & 0xffu) * LV * 32 + lane;
+          for (int v = 0; v < LV; ++v) Xw[v * 32 + lane] = src[(size_t)v * 32];
+        }
+        for (int t = 1; t < p.nops; ++t) {
+          const uint32_t op = p.ops[t];
+          for (uint32_t s = op >> 8; s > 0; --s) mont_call<K, M, MONT_SQR>(io);
+          const uint32_t idx = op & 0xffu;
+          if (idx != 0xffu) {
+            io.Y = idx == 0xfeu ? ONErep : tab + (size_t)idx * LV * 32 + lane;
+            mont_call<K, M, MONT_MUL>(io);
+          }
         }
       }
     }
